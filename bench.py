@@ -83,7 +83,28 @@ def parse():
                     help="cudaProfilerStart/Stop around the timed steps (for ncu --profile-from-start off)")
     ap.add_argument("--no-graph", dest="graph", action="store_false",
                     help="launch every kernel from the host instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the main tier computed as DIR/<name>.npy: the sampler state after the "
+                         "last timed step (rank 0's shard) and the end-to-end samples")
     return ap.parse_args()
+
+
+DUMP_LIMIT = 64 * 10**6
+
+
+def dump_outputs(path, arrays, limit=DUMP_LIMIT):
+    """Writes every array as ``path/<name>.npy`` in float64 or float32.  When the files would come to
+    more than ``limit`` bytes, each keeps a fixed, seeded sample of its leading (batch) rows."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    budget = limit - 4096 * len(arrays)          # room for the .npy headers
+    for name, v in arrays.items():
+        if total > budget:
+            keep = max(1, v.shape[0] * budget // total)
+            v = v[np.sort(np.random.default_rng(0).choice(v.shape[0], keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), v)
 
 
 def peaks():
@@ -286,6 +307,8 @@ def measure_tier(args, precision, ctx):
         dist.barrier()
     ms_total = max_over_ranks(e0.elapsed_time(e1), dev)
     clk = clocks.stop() if clocks is not None else None
+    # copied now: the update roofline below runs the update kernel in place on `state`
+    outputs = {"state": state.cpu().numpy()} if args.dump_outputs else {}
     ms_per_step = ms_total / args.steps
     value = B * world / (NFE * ms_per_step * 1e-3)
     # first-half-step launch + per step (program + fused update)
@@ -370,6 +393,8 @@ def measure_tier(args, precision, ctx):
                "d2h_bytes_per_step": int(host.numel() * host.element_size()),
                "seconds": dt, "nfe": args.e2e_nfe, "api": "SSCSSampler.sample + gather_samples",
                "finite": bool(torch.isfinite(host).all().item())}
+        if args.dump_outputs:
+            outputs["samples"] = host.numpy()
     return {"precision": precision, "dtype": TIER_DTYPE[precision], "note": TIER_NOTE[precision],
             "value": value, "ms_per_step": ms_per_step, "e2e": e2e, "roofline": roof, "clocks": clk,
             "gpu_launches": launches, "finite": finite, "engines": dict(plan.engine_count),
@@ -377,7 +402,7 @@ def measure_tier(args, precision, ctx):
             "per_kernel_ms": {k: round(v["ms"] / total_ms * ms_per_step, 4) for k, v in prof.items()},
             "conv_classes": {k: {"n": v["n"], "ms": round(v["ms"], 4), "tflops": round(v["tflops"], 1)}
                              for k, v in sorted(conv_classes.items(), key=lambda kv: -kv[1]["ms"])},
-            "_state": state, "_plan": plan}
+            "_state": state, "_plan": plan, "_outputs": outputs}
 
 
 def gpu_eager_baseline(cfg, sde_cfg_B, dev, steps=2):
@@ -521,6 +546,8 @@ def main_b200(args):
         }
         if other is not None:
             line[other["precision"] + "_path"] = other
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, main["_outputs"])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,73 +1,97 @@
-"""CPU, build container only: the oracle against the UNMODIFIED reference imported from
-/root/reference (skipped where the reference is absent, e.g. on the GPU box)."""
+"""CPU: the oracle against the UNMODIFIED reference, through outputs of the reference stored under
+``tests/golden/`` (written by ``oracle/make_golden.py`` from the reference's own modules and samplers)."""
+import json
+import types
+
 import numpy as np
 import pytest
 import torch
 
 from oracle import psld_oracle as O
-from oracle.ref_loader import NoiseBank, load_reference, reference_available, reference_time_grid
 from oracle.weights import fill_state_dict, noise_bank, prior
 from psld_b200 import NCSNpp, tiny_config
+from _net import fake_score
+from test_gpu_sampler import _golden_cfg
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="/root/reference not present")
 
-
-def test_state_dict_contract():
+def test_state_dict_contract(golden_dir):
     """psld_b200.NCSNpp exposes exactly the reference's parameter names and shapes."""
-    R = load_reference()
-    for cfg in (tiny_config(),):
-        ref = R.NCSNpp(cfg).state_dict()
+    ref = json.load(open(f"{golden_dir}/state_dict_contract.json"))
+    for name, cfg in (("tiny", tiny_config()),):
         mine = NCSNpp(cfg).state_dict()
-        assert list(ref.keys()) == list(mine.keys())
-        for k in ref:
-            assert tuple(ref[k].shape) == tuple(mine[k].shape), k
+        assert list(ref[name].keys()) == list(mine.keys())
+        for k in ref[name]:
+            assert tuple(ref[name][k]) == tuple(mine[k].shape), k
 
 
-def test_forward_bit_exact():
-    R = load_reference()
+def test_forward_bit_exact(golden_dir):
+    """The oracle forward is the reference forward op for op.  CPU convolutions partition their
+    sums by thread count, so the oracle runs with the 8 threads the fixture was written with."""
+    g = np.load(f"{golden_dir}/forward_tiny.npz")
     cfg = tiny_config()
-    net = R.NCSNpp(cfg).eval()
-    sd = fill_state_dict({k: tuple(v.shape) for k, v in net.state_dict().items()}, 3)
-    net.load_state_dict(sd)
-    x = torch.randn(2, 6, 32, 32, generator=torch.Generator().manual_seed(0))
-    t = torch.tensor([0.9, 0.004])
-    with torch.no_grad():
-        y = net(x, t)
-    assert torch.equal(y, O.ncsnpp_forward(cfg, sd, x, t))
+    sd = fill_state_dict({k: tuple(v.shape) for k, v in NCSNpp(cfg).state_dict().items()}, int(g["seed"]))
+    threads = torch.get_num_threads()
+    torch.set_num_threads(8)
+    try:
+        y = O.ncsnpp_forward(cfg, sd, torch.from_numpy(g["x"]), torch.from_numpy(g["t"]))
+    finally:
+        torch.set_num_threads(threads)
+    assert torch.equal(y, torch.from_numpy(g["y"]))
 
 
 @pytest.mark.parametrize("kind", ["sscs_sde", "em_sde"])
-def test_sampler(kind):
-    R = load_reference()
-    cfg = tiny_config(sampler=kind, n_discrete_steps=12)
-    cfg.data.image_size = 8
-    fake = lambda u, t: torch.tanh(u) * t.view(-1, 1, 1, 1)
-    sde = R.PSLD(cfg)
-    ts, n = reference_time_grid(cfg)
-    u0 = prior((2, 3, 8, 8), 0.5, 5)
-    nb = noise_bank((2 if kind == "sscs_sde" else 1) * n, (2, 6, 8, 8), 6)
-    with NoiseBank(nb):
-        ref = R.get_module("samplers", kind)(cfg, sde, fake).sample(u0.clone(), ts, n)
+def test_sampler(golden_dir, kind):
+    """The reference's own SSCS / EM sampler with a stand-in score, step by step: per-step sum,
+    |sum|, max|.| and sum of squares of the state, and the final samples."""
+    tag = kind.split("_")[0] + "_fake_uniform"
+    g = np.load(f"{golden_dir}/sampler_{tag}.npz")
+    cfg = _golden_cfg(tag)
+    ts, n = O.time_grid(cfg)
+    B = int(g["B"])
+    u0 = prior((B, 3, 8, 8), float(np.sqrt(O.PSLDScalars(cfg).m)), 1)
+    nb = noise_bank((2 if kind == "sscs_sde" else 1) * n, (B, 6, 8, 8), 2)
+    stats = []
+    rec = lambda i, u: stats.append([u.sum().item(), u.abs().sum().item(), u.abs().max().item(),
+                                     (u.double() ** 2).sum().item()])
     fn = O.sscs_sample if kind == "sscs_sde" else O.em_sample
-    out = fn(cfg, fake, u0, O.time_grid(cfg)[0], n, nb)
+    out = fn(cfg, fake_score, u0, ts, n, nb, record=rec)
     # 5e-7: the reference does its first step partly in fp32 (fp32 prior x python scalars), the
     # oracle promotes the prior to fp64 first (documented in oracle/psld_oracle.py)
+    ref = torch.from_numpy(g["final"])
     assert (out - ref).abs().max() <= 5e-7 * ref.abs().max()
+    got, want = np.asarray(stats), g["stats"]
+    assert got.shape == want.shape
+    assert np.all(np.abs(got[:, 0] - want[:, 0]) <= 5e-7 * want[:, 1])
+    np.testing.assert_allclose(got[:, 1:], want[:, 1:], rtol=5e-7, atol=0)
+
+
+def _reference_util():
+    """The reference's registry (``main/util.py:33-62``): the ``_MODULES`` table holding the
+    reference's own names, and ``get_module``."""
+    util = types.ModuleType("util")
+    util._MODULES = {"samplers": {"sscs_sde": type("SSCSSampler", (), {}),
+                                  "em_sde": type("EulerMaruyamaSampler", (), {})},
+                     "score_fn": {"ncsnpp": type("NCSNpp", (), {})}}
+
+    def get_module(category, name):
+        module = util._MODULES.get(category, dict()).get(name, None)
+        if module is None:
+            raise ValueError(f"No module named `{name}` found in category: `{category}`")
+        return module
+
+    util.get_module = get_module
+    return util
 
 
 def test_registry_install():
     """install() publishes the B200 classes into the reference registry (util.py:33-62)."""
-    R = load_reference()
     import psld_b200
-    reg = psld_b200.install(R.util)
-    assert R.get_module("samplers", "sscs_sde_b200") is psld_b200.SSCSSampler
-    assert R.get_module("score_fn", "ncsnpp_b200") is psld_b200.NCSNpp
-    assert R.get_module("samplers", "sscs_sde") is not psld_b200.SSCSSampler   # no override
-    keep = dict(reg["samplers"])
-    try:
-        psld_b200.install(R.util, override=True)
-        assert R.get_module("samplers", "sscs_sde") is psld_b200.SSCSSampler
-        assert R.get_module("score_fn", "ncsnpp") is psld_b200.NCSNpp
-    finally:
-        reg["samplers"].update(keep)
-        reg["score_fn"]["ncsnpp"] = R.NCSNpp
+    util = _reference_util()
+    ref_sscs = util.get_module("samplers", "sscs_sde")
+    psld_b200.install(util)
+    assert util.get_module("samplers", "sscs_sde_b200") is psld_b200.SSCSSampler
+    assert util.get_module("score_fn", "ncsnpp_b200") is psld_b200.NCSNpp
+    assert util.get_module("samplers", "sscs_sde") is ref_sscs                  # no override
+    psld_b200.install(util, override=True)
+    assert util.get_module("samplers", "sscs_sde") is psld_b200.SSCSSampler
+    assert util.get_module("score_fn", "ncsnpp") is psld_b200.NCSNpp
