@@ -446,17 +446,11 @@ extern "C" __attribute__((visibility("default"))) int psld_debug_attn_trace(long
 
 // ---------------------------------------------------------------- host side
 static int encode_qkv_map(CUtensorMap* tm, const void* ptr, int N, int HW, int C3, int rows) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
-  cuuint64_t dims[3] = {(cuuint64_t)C3, (cuuint64_t)HW, (cuuint64_t)N};
-  cuuint64_t strides[2] = {(cuuint64_t)C3 * 2, (cuuint64_t)HW * C3 * 2};
-  cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(ptr), dims, strides,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(qkv) failed: %d", (int)r); return PSLD_ECUDA; }
-  return PSLD_OK;
+  const cuuint64_t dims[3] = {(cuuint64_t)C3, (cuuint64_t)HW, (cuuint64_t)N};
+  const cuuint64_t strides[2] = {(cuuint64_t)C3 * 2, (cuuint64_t)HW * C3 * 2};
+  const cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  return encode_bf16_map(tm, ptr, 3, dims, strides, box, estr, "qkv");
 }
 
 int prepare_attn_tc(psld_op& op) {
@@ -488,16 +482,9 @@ int prepare_attn_tc(psld_op& op) {
   st->proj = op.i[PSLD_ATTN_PROJ] != 0;
   if (st->proj) {
     if (HW % 128 || !op.in[1] || !op.in[3]) { delete st; return unsupported("fused projection needs HW %% 128 == 0, weight and residual"); }
-    EncodeTiledFn enc = get_encode_fn();
-    cuuint64_t dims[2] = {(cuuint64_t)C, (cuuint64_t)(cm * C)};      // split: planes [2][C out, C in]
-    cuuint64_t strides[1] = {(cuuint64_t)C * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)(C < 128 ? C : 128)};        // <=128-row output tiles
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc ? enc(&st->tw, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(op.in[1]), dims,
-                           strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE)
-                     : CUDA_ERROR_UNKNOWN;
-    if (r != CUDA_SUCCESS) { delete st; set_error("cuTensorMapEncodeTiled(proj weight) failed: %d", (int)r); return PSLD_ECUDA; }
+    // W3 [C out, C in] (split: planes [2][C out, C in]) in <=128-row output tiles
+    rc = encode_w_map(&st->tw, op.in[1], cm * C, C, C < 128 ? C : 128);
+    if (rc != PSLD_OK) { delete st; return rc; }
     ConvTcParams& e = st->p.ep;
     e = ConvTcParams{};
     e.bias = (const float*)op.in[2];

@@ -7,7 +7,6 @@
 // incurs 9 `.item()` syncs per SSCS step, SURVEY.md §3.1).
 
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -21,14 +20,6 @@ void set_error(const char* fmt, ...) {
   va_start(ap, fmt);
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
-}
-
-bool pdl_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("PSLD_PDL");
-    return !(e && e[0] == '0');
-  }();
-  return on;
 }
 
 static int op_launch_count(const psld_op& op) {

@@ -41,7 +41,7 @@ static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 // weight fetch a visible share of a step).  Contract: a kernel launched through launch_pdl()
 // executes pdl_wait() before it reads or writes ANY global memory another kernel may touch
 // (weights / constant tables are exempt); kernels that fit the GPU in a single wave may call
-// pdl_launch_dependents() early.  PSLD_PDL=0 launches everything fully serialized.
+// pdl_launch_dependents() early.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() {
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
@@ -50,13 +50,7 @@ __device__ __forceinline__ void pdl_launch_dependents() {
 // the hardware once EVERY block of this grid has started (so it never competes with unscheduled
 // blocks), its prologue (barrier init, TMEM allocation, descriptor prefetch) and launch latency then
 // overlap this kernel's last wave; correctness still rests on the dependent's pdl_wait().
-// -DPSLD_NO_EARLY_TRIGGER restores the implicit trigger at exit (A/B switch).
-__device__ __forceinline__ void pdl_trigger_early() {
-#ifndef PSLD_NO_EARLY_TRIGGER
-  pdl_launch_dependents();
-#endif
-}
-bool pdl_enabled();
+__device__ __forceinline__ void pdl_trigger_early() { pdl_launch_dependents(); }
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
@@ -75,11 +69,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
     attr[n].val.clusterDim.z = 1;
     ++n;
   }
-  if (pdl_enabled()) {
-    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[n].val.programmaticStreamSerializationAllowed = 1;
-    ++n;
-  }
+  attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[n].val.programmaticStreamSerializationAllowed = 1;
+  ++n;
   cfg.attrs = attr;
   cfg.numAttrs = n;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);

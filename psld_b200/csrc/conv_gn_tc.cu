@@ -20,14 +20,13 @@
 // An optional 1x1 "extension" over a second, un-normalised input (the block's Conv_2 shortcut)
 // adds one-tap chunks that bypass the transform.  In THIS (bf16) kernel they travel through the two
 // big operand sets, whose latency a one-tap chunk cannot hide, so the bf16 plan keeps shortcut blocks
-// on conv_tc + an apply pass (PSLD_TC_FUSE_GN_EXT=1 forces them here); the split-bf16 kernel below
+// on conv_tc + an apply pass; the split-bf16 kernel below
 // streams them through a ring of their own and takes them by default.
 //
 // Warps (640 threads): 0 = raw-tile TMA, 1 = MMA issuer (leader CTA) + TMEM allocator,
 // 2 = weight TMA, 3 idle, 4..11 = epilogue (shared with conv_tc), 12..19 = transform.
 
 #include <cuda.h>
-#include <stdlib.h>
 
 #include <new>
 
@@ -813,31 +812,11 @@ conv_gn_x3_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constan
 
 // ---------------------------------------------------------------- host side
 static int encode_raw_map(CUtensorMap* tm, const void* ptr, int N, int H, int W, int C, int rows_y) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)W, (cuuint32_t)rows_y, 1};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(raw tile) failed: %d", (int)r); return PSLD_ECUDA; }
-  return PSLD_OK;
-}
-
-static int encode_w_half_map(CUtensorMap* tm, const void* ptr, int Cout, int K, int rows) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)Cout};
-  cuuint64_t strides[1] = {(cuuint64_t)K * 2};
-  cuuint32_t box[2] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(weight) failed: %d", (int)r); return PSLD_ECUDA; }
-  return PSLD_OK;
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
+  const cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)W, (cuuint32_t)rows_y, 1};
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  return encode_bf16_map(tm, ptr, 4, dims, strides, box, estr, "raw tile");
 }
 
 // Returns PSLD_EUNSUPPORTED when the shape must take the unfused route (GroupNorm apply + conv_tc).
@@ -850,8 +829,6 @@ int prepare_conv_gn_tc(psld_op& op) {
               W, C1, C2, Cout, KS);
     return PSLD_EUNSUPPORTED;
   };
-  static const int env = [] { const char* e = getenv("PSLD_TC_FUSE_GN"); return e ? atoi(e) : 1; }();
-  if (!env) return unsupported("disabled by PSLD_TC_FUSE_GN=0");
   // network head (ncsnpp.py:430): fp32 NCHW output, first f[1] channels of a zero-padded Cout
   const bool head = op.i[PSLD_CONV_OUT_LAYOUT] == PSLD_NCHW && op.i[PSLD_CONV_OUT_DTYPE] == PSLD_F32;
   const int adt = op.i[PSLD_CONV_IN_DTYPE];
@@ -879,12 +856,6 @@ int prepare_conv_gn_tc(psld_op& op) {
   if (rows_in > GN_MAX_ROWS) return unsupported("tile rows");
   const int64_t m_tiles = (int64_t)N * (H / BH);
   if (m_tiles < 2) return unsupported("single tile");
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-    cudaGetLastError();
-    sms = 148;
-  }
   ConvGnState* st = new (std::nothrow) ConvGnState();
   if (!st) { set_error("conv_gn_tc: out of host memory"); return PSLD_ECUDA; }
   st->x3 = x3;
@@ -908,46 +879,24 @@ int prepare_conv_gn_tc(psld_op& op) {
                          : encode_raw_map(&st->e2, op.in[0], N, H, W, cm * C1, BH + 2);
   const int K = 9 * (C1 + C2) + (ext ? E1 + E2 : 0);
   // split bf16: weight planes [2][Cout, K] seen as one [2*Cout, K] matrix
-  if (rc == PSLD_OK) rc = encode_w_half_map(&st->b, op.in[4], cm * Cout, K, block_n / 2);
+  if (rc == PSLD_OK) rc = encode_w_map(&st->b, op.in[4], cm * Cout, K, block_n / 2);
   if (rc != PSLD_OK) { delete st; return rc; }
   ConvGnParams& g = st->p;
   ConvTcParams& p = g.c;
-  p.bias = (const float*)op.in[5];
-  p.temb = (const float*)op.in[3];
-  p.res = (const __nv_bfloat16*)op.in[2];
-  p.y = head ? nullptr : (__nv_bfloat16*)op.out[0];
-  p.y_nchw = head ? (float*)op.out[0] : nullptr;
-  p.cout_valid = head ? (int)op.f[1] : Cout;
-  p.mg_stats = (double*)op.out[1];
-  p.scale = op.f[0];
-  p.temb_off = op.i[PSLD_CONV_TEMB_OFF];
-  p.temb_bstride = op.i[PSLD_CONV_TEMB_BSTRIDE];
-  p.H = H; p.W = W; p.HW = H * W; p.Cout = Cout;
-  p.stride = 1; p.pad = 1;
-  p.BH = BH; p.BN_img = 1; p.tiles_y = H / BH;
-  p.kchunks1 = C1 / TC_BLOCK_K; p.kchunks = (C1 + C2) / TC_BLOCK_K;
-  p.taps = 9; p.KS = 3;
-  p.ext_kchunks1 = ext ? E1 / TC_BLOCK_K : 0;
-  p.ext_kchunks = ext ? (E1 + E2) / TC_BLOCK_K : 0;
-  p.block_n = block_n; p.n_tiles_n = Cout / block_n;
-  p.M = (int64_t)N * H * W;
+  tc_conv_params(p, op, head, H, W, BH, 1, block_n);
   p.num_tiles = (int)(((m_tiles + 1) / 2) * p.n_tiles_n);
-  p.lo1 = C1; p.lo2 = C2; p.loe1 = E1; p.loe2 = E2; p.w_lo_rows = Cout;
   g.affine = (const float*)op.in[6];
   g.cin = C1 + C2;
   g.silu = op.i[PSLD_CONV_GN_SILU];
   g.rows_in = rows_in;
   g.w_shift = W == 32 ? 5 : 4;
   g.n_images = N;
-  const int pairs = sms / 2;
+  const int pairs = sm_count() / 2;
   st->b2 = st->b;
-  {
-    static const int split_env = [] { const char* e = getenv("PSLD_TC_TAIL_SPLIT"); return e ? atoi(e) : 1; }();
-    const int ns = tc_plan_tail_split(p, pairs, 64, split_env && !head);
-    if (ns > 1) {
-      rc = encode_w_half_map(&st->b2, op.in[4], cm * Cout, K, block_n / ns / 2);
-      if (rc != PSLD_OK) { delete st; return rc; }
-    }
+  const int ns = tc_plan_tail_split(p, pairs, 64, !head);
+  if (ns > 1) {
+    rc = encode_w_map(&st->b2, op.in[4], cm * Cout, K, block_n / ns / 2);
+    if (rc != PSLD_OK) { delete st; return rc; }
   }
   st->grid = 2 * (p.num_virtual < pairs ? p.num_virtual : pairs);
   static bool attr_set = false;

@@ -36,8 +36,6 @@
 
 #include <cuda.h>
 
-#include <stdlib.h>
-
 #include <new>
 
 #include "common.cuh"
@@ -330,32 +328,12 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
 // (split bf16: C = 2 x channels, the row holds [hi | lo])
 static int encode_act_map(CUtensorMap* tm, const void* ptr, int N, int H, int W, int C, int OW,
                           int BH, int BN_img, int stride) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)(OW * stride), (cuuint32_t)(BH * stride),
-                       (cuuint32_t)BN_img};
-  cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(ptr), dims, strides,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(activation) failed: %d", (int)r); return PSLD_ECUDA; }
-  return PSLD_OK;
-}
-
-static int encode_w_map(CUtensorMap* tm, const void* ptr, int Cout, int K, int block_n) {
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
-  cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)Cout};
-  cuuint64_t strides[1] = {(cuuint64_t)K * 2};
-  cuuint32_t box[2] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)block_n};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides,
-                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(weight) failed: %d", (int)r); return PSLD_ECUDA; }
-  return PSLD_OK;
+  const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
+  const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
+  const cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)(OW * stride), (cuuint32_t)(BH * stride),
+                             (cuuint32_t)BN_img};
+  const cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
+  return encode_bf16_map(tm, ptr, 4, dims, strides, box, estr, "activation");
 }
 
 static bool is_pow2(int v) { return v > 0 && (v & (v - 1)) == 0; }
@@ -399,6 +377,9 @@ int prepare_conv_tc(psld_op& op) {
     set_error("conv_tc: null pointer");
     return PSLD_EINVAL;
   }
+  // N tile = the widest that divides Cout.  (Measured: narrowing to N=128 to fix the wave
+  // quantisation of the 16x16 layers - 7 half rounds instead of 4 - is a net loss, 2.0 -> 2.8 ms:
+  // k-blocks then retire every 256 cycles and the TMA issue loops cannot keep up.)
   int block_n = 0;
   for (int cand : {256, 128, 64, 32})
     if (Cout % cand == 0) { block_n = cand; break; }
@@ -407,30 +388,10 @@ int prepare_conv_tc(psld_op& op) {
   const int BN_img = 128 / (OW * BH);
   if (BN_img > 256) return unsupported("image too small");
 
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
-    cudaGetLastError();
-    sms = 148;
-  }
-  // 2-CTA pairs whenever there are at least two M tiles (PSLD_TC_PAIR=0 forces the 1-CTA kernel)
+  const int sms = sm_count();
+  // 2-CTA pairs whenever there are at least two M tiles
   const int64_t m_tiles_all = (int64_t)((N + BN_img - 1) / BN_img) * (OH / BH);
-  static const int pair_env = [] {
-    const char* e = getenv("PSLD_TC_PAIR");
-    return e ? atoi(e) : 1;
-  }();
-  const bool pair = pair_env != 0 && m_tiles_all >= 2 && sms >= 2;
-  // N tile = the widest that divides Cout.  (Measured: narrowing to N=128 to fix the wave
-  // quantisation of the 16x16 layers - 7 half rounds instead of 4 - is a net loss, 2.0 -> 2.8 ms:
-  // k-blocks then retire every 256 cycles and the TMA issue loops cannot keep up.)
-  // PSLD_TC_BLOCK_N overrides for experiments.
-  {
-    static const int bn_env = [] {
-      const char* e = getenv("PSLD_TC_BLOCK_N");
-      return e ? atoi(e) : 0;
-    }();
-    if (bn_env > 0 && bn_env <= block_n && Cout % bn_env == 0 && bn_env % 32 == 0) block_n = bn_env;
-  }
+  const bool pair = m_tiles_all >= 2 && sms >= 2;
   ConvTcState* st = new (std::nothrow) ConvTcState();
   if (!st) { set_error("conv_tc: out of host memory"); return PSLD_ECUDA; }
   int rc = encode_act_map(&st->a1, op.in[0], N, H, W, cm * C1, OW, BH, BN_img, stride);
@@ -456,31 +417,12 @@ int prepare_conv_tc(psld_op& op) {
   st->b2 = st->b;
 
   ConvTcParams& p = st->p;
-  p.bias = (const float*)op.in[5];
-  p.temb = (const float*)op.in[3];
-  p.res = (const __nv_bfloat16*)op.in[2];
-  p.y = head ? nullptr : (__nv_bfloat16*)op.out[0];
-  p.y_nchw = head ? (float*)op.out[0] : nullptr;
-  p.cout_valid = head ? (int)op.f[1] : Cout;
-  p.mg_stats = (double*)op.out[1];
+  tc_conv_params(p, op, head, OH, OW, BH, BN_img, block_n);
   if (p.mg_stats && (head || (OH * OW) % 32 != 0)) {
     delete st;
     set_error("conv_tc: micro-group stats need NHWC bf16 output and H*W %% 32 == 0");
     return PSLD_EINVAL;
   }
-  p.scale = op.f[0];
-  p.temb_off = op.i[PSLD_CONV_TEMB_OFF];
-  p.temb_bstride = op.i[PSLD_CONV_TEMB_BSTRIDE];
-  p.H = OH; p.W = OW; p.HW = OH * OW; p.Cout = Cout;
-  p.stride = stride; p.pad = pad;
-  p.BH = BH; p.BN_img = BN_img; p.tiles_y = OH / BH;
-  p.kchunks1 = C1 / TC_BLOCK_K; p.kchunks = (C1 + C2) / TC_BLOCK_K;
-  p.taps = KS * KS; p.KS = KS;
-  p.ext_kchunks1 = ext ? E1 / TC_BLOCK_K : 0;
-  p.ext_kchunks = ext ? (E1 + E2) / TC_BLOCK_K : 0;
-  p.block_n = block_n; p.n_tiles_n = Cout / block_n;
-  p.M = (int64_t)N * OH * OW;
-  p.lo1 = C1; p.lo2 = C2; p.loe1 = E1; p.loe2 = E2; p.w_lo_rows = Cout;
   st->x3 = x3;
   const int64_t m_tiles = (int64_t)((N + BN_img - 1) / BN_img) * p.tiles_y;
   const int64_t m_units = pair ? (m_tiles + 1) / 2 : m_tiles;
@@ -488,18 +430,12 @@ int prepare_conv_tc(psld_op& op) {
   st->pair = pair;
   // ---- last partial round: split its units along N when that lets the idle clusters share the work
   // (16x16 CIFAR layers at B = 256: 256 tile pairs over 74 clusters = 3 rounds + 34 units; as 68
-  // half-N units the tail costs half a round: 4 -> 3.5 rounds).  PSLD_TC_TAIL_SPLIT=0 disables it.
-  {
-    static const int split_env = [] {
-      const char* e = getenv("PSLD_TC_TAIL_SPLIT");
-      return e ? atoi(e) : 1;
-    }();
-    const int best = tc_plan_tail_split(p, pair ? sms / 2 : sms, 64, split_env && !head);
-    if (best > 1) {
-      const int sub = block_n / best;
-      rc = encode_w_map(&st->b2, op.in[4], cm * Cout, K, pair ? sub / 2 : sub);
-      if (rc != PSLD_OK) { delete st; return rc; }
-    }
+  // half-N units the tail costs half a round: 4 -> 3.5 rounds).
+  const int best = tc_plan_tail_split(p, pair ? sms / 2 : sms, 64, !head);
+  if (best > 1) {
+    const int sub = block_n / best;
+    rc = encode_w_map(&st->b2, op.in[4], cm * Cout, K, pair ? sub / 2 : sub);
+    if (rc != PSLD_OK) { delete st; return rc; }
   }
   if (pair) {
     const int pairs = sms / 2;

@@ -578,4 +578,56 @@ __device__ __forceinline__ void tc_epilogue_tile(const ConvTcParams& p, uint32_t
   }  // legacy (non-staged) path
 }
 
+// Host: [rows, K] bf16 weight matrix, K contiguous (split bf16: the planes [2][Cout, K] as one
+// [2*Cout, K] matrix); box = one 64-wide K chunk x box_rows rows.
+static inline int encode_w_map(CUtensorMap* tm, const void* ptr, int rows, int K, int box_rows) {
+  const cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)K * 2};
+  const cuuint32_t box[2] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)box_rows};
+  const cuuint32_t estr[2] = {1, 1};
+  return encode_bf16_map(tm, ptr, 2, dims, strides, box, estr, "weight");
+}
+
+// Host: SMs of the current device (148 if the query fails).
+static inline int sm_count() {
+  int dev = 0, sms = 148;
+  cudaGetDevice(&dev);
+  if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) {
+    cudaGetLastError();
+    sms = 148;
+  }
+  return sms;
+}
+
+// Host: the ConvTcParams fields that follow from a validated conv op record and its tiling (OH x OW
+// output, M tiles of BH rows x BN_img images, N tiles of block_n channels).  num_tiles and the tail
+// split are left to the caller.
+static inline void tc_conv_params(ConvTcParams& p, const psld_op& op, bool head, int OH, int OW, int BH,
+                                  int BN_img, int block_n) {
+  const int N = op.i[PSLD_CONV_N], C1 = op.i[PSLD_CONV_C1], C2 = op.i[PSLD_CONV_C2];
+  const int Cout = op.i[PSLD_CONV_COUT], KS = op.i[PSLD_CONV_KS];
+  const int E1 = op.i[PSLD_CONV_EXT_C1], E2 = op.i[PSLD_CONV_EXT_C2];
+  const bool ext = op.in[8] != nullptr && E1 > 0;
+  p.bias = (const float*)op.in[5];
+  p.temb = (const float*)op.in[3];
+  p.res = (const __nv_bfloat16*)op.in[2];
+  p.y = head ? nullptr : (__nv_bfloat16*)op.out[0];
+  p.y_nchw = head ? (float*)op.out[0] : nullptr;
+  p.cout_valid = head ? (int)op.f[1] : Cout;
+  p.mg_stats = (double*)op.out[1];
+  p.scale = op.f[0];
+  p.temb_off = op.i[PSLD_CONV_TEMB_OFF];
+  p.temb_bstride = op.i[PSLD_CONV_TEMB_BSTRIDE];
+  p.H = OH; p.W = OW; p.HW = OH * OW; p.Cout = Cout;
+  p.stride = op.i[PSLD_CONV_STRIDE]; p.pad = op.i[PSLD_CONV_PAD];
+  p.BH = BH; p.BN_img = BN_img; p.tiles_y = OH / BH;
+  p.kchunks1 = C1 / TC_BLOCK_K; p.kchunks = (C1 + C2) / TC_BLOCK_K;
+  p.taps = KS * KS; p.KS = KS;
+  p.ext_kchunks1 = ext ? E1 / TC_BLOCK_K : 0;
+  p.ext_kchunks = ext ? (E1 + E2) / TC_BLOCK_K : 0;
+  p.block_n = block_n; p.n_tiles_n = Cout / block_n;
+  p.M = (int64_t)N * OH * OW;
+  p.lo1 = C1; p.lo2 = C2; p.loe1 = E1; p.loe2 = E2; p.w_lo_rows = Cout;
+}
+
 }  // namespace psld

@@ -40,9 +40,9 @@ struct Philox {
   // 4 standard normals from one draw (Box-Muller on two uniform pairs).  The radius uses the
   // full-accuracy logf (the tail is where a relative error of the logarithm would show); the angle
   // is drawn on [-pi, pi), the interval on which sin.approx / cos.approx are specified to 2^-21.4
-  // absolute error, i.e. below the fp32 rounding of the state the noise is added to
-  // (-DPSLD_RNG_EXACT_TRIG switches to sincospif; it costs 96 more instructions per 4 pairs and
-  // takes the fused update at 2^24 pairs from bandwidth-bound to issue-bound).  The radius uniform
+  // absolute error, i.e. below the fp32 rounding of the state the noise is added to (sincospif
+  // would cost 96 more instructions per 4 pairs and take the fused update at 2^24 pairs from
+  // bandwidth-bound to issue-bound).  The radius uniform
   // is (n + 0.5) 2^-32 in (0, 1): the tail reaches sqrt(-2 ln 2^-33) = 6.76 sigma.  Statistical
   // checks on 2.5e7 draws per stream: tests/test_gpu_kernels.py::test_philox_normal_quality.
   static __device__ __forceinline__ float4 normal4(uint64_t seed, uint64_t stream, uint64_t index) {
@@ -52,21 +52,12 @@ struct Philox {
     float u2 = ((float)r.z + 0.5f) * k, u3 = (float)r.w * k;
     u0 = fminf(u0, 0.99999994f);
     u2 = fminf(u2, 0.99999994f);
-#ifdef PSLD_RNG_FAST_LOG
-    float ra = sqrtf(-2.0f * __logf(u0)), rb = sqrtf(-2.0f * __logf(u2));
-#else
     float ra = sqrtf(-2.0f * logf(u0)), rb = sqrtf(-2.0f * logf(u2));
-#endif
     float sa, ca, sb, cb;
-#ifdef PSLD_RNG_EXACT_TRIG
-    sincospif(2.0f * u1, &sa, &ca);
-    sincospif(2.0f * u3, &sb, &cb);
-#else
     // angle uniform on [-pi, pi): the range where sin.approx / cos.approx are specified to
     // 2^-21.4 ABSOLUTE error (the former code fed them [0, 2 pi), outside that range)
     __sincosf(6.283185307179586f * (u1 - 0.5f), &sa, &ca);
     __sincosf(6.283185307179586f * (u3 - 0.5f), &sb, &cb);
-#endif
     return make_float4(ra * ca, ra * sa, rb * cb, rb * sb);
   }
 };

@@ -150,5 +150,19 @@ static inline EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
+// Every operand map of the tensor-core kernels: bf16 elements, 128-byte swizzle (the UMMA operand
+// layout), 256-byte L2 promotion, out-of-bounds boxes zero-filled.  `what` names the map in the
+// error message.
+static inline int encode_bf16_map(CUtensorMap* tm, const void* ptr, int rank, const cuuint64_t* dims,
+                                  const cuuint64_t* strides, const cuuint32_t* box,
+                                  const cuuint32_t* estr, const char* what) {
+  EncodeTiledFn enc = get_encode_fn();
+  if (!enc) { set_error("cuTensorMapEncodeTiled entry point unavailable"); return PSLD_ECUDA; }
+  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(ptr), dims,
+                   strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled(%s) failed: %d", what, (int)r); return PSLD_ECUDA; }
+  return PSLD_OK;
+}
 
 }  // namespace psld

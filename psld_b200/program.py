@@ -22,7 +22,6 @@ Fusions relative to the reference's eager graph (SURVEY.md §3.2, §7.3-4):
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 import torch
@@ -68,10 +67,6 @@ class Plan:
         self.mg = {}            # data_ptr of an activation -> its GroupNorm statistics accumulator
         self.stat_chunks = []   # f64 arenas the accumulators are carved from (zeroed by OP_ZERO)
         self.stat_used = []
-        self.fused_stats = True
-        self.fuse_gn = True
-        self.fuse_gn_residual = False   # force GroupNorm_1 -> Conv_1 fusion (default: PSLD_TC_FUSE_GN1)
-        self.fuse_shortcut = True       # Conv_2 (1x1 shortcut) as extra K-blocks of Conv_1
         self.temb_op = -1
         self._build()
         self.n_ops = len(self.ops)
@@ -97,9 +92,7 @@ class Plan:
     def _gn_fusable(self, x1, x2, cout):
         """Host mirror of prepare_conv_gn_tc (csrc/conv_gn_tc.cu): can act(GroupNorm(x)) -> conv3x3
         run as ONE kernel that normalises its input tile in shared memory?"""
-        if not self.tc or not self.fuse_gn or os.environ.get("PSLD_TC_FUSE_GN", "1") == "0":
-            return False
-        if self.x3 and os.environ.get("PSLD_X3_FUSE_GN", "1") == "0":
+        if not self.tc:
             return False
         N, H, W, C1 = x1.shape
         C2 = x2.shape[-1] if x2 is not None else 0
@@ -111,7 +104,7 @@ class Plan:
 
     def _ext_fusable(self, b, e1, e2, cout):
         """Can Conv_2 (1x1 shortcut over e = cat(e1, e2)) ride along Conv_1's MMA stream?"""
-        if not self.tc or not self.fuse_shortcut:
+        if not self.tc:
             return False
         N, H, W, Cb = b.shape
         E1 = e1.shape[-1]
@@ -159,6 +152,38 @@ class Plan:
         t = t.detach().to(device=self.dev, dtype=dtype).contiguous()
         self.keep.append(t)
         return t
+
+    def _w_bf16(self, w):
+        """fp32 weight [rows, K] as a tensor-core operand: bf16, or for split-bf16 plans the planes
+        [2][rows, K] with hi = rn(w), lo = rn(w - hi)."""
+        if self.x3:
+            hi = w.to(torch.bfloat16)
+            w = torch.cat([hi, (w - hi.to(torch.float32)).to(torch.bfloat16)], 0)
+        return self._w(w, torch.bfloat16)
+
+    def _pack_tc_conv(self, op, w, b32, ext, cout_pad):
+        """Weight and bias of a tensor-core convolution: w [Cout, Cin, ks, ks] becomes [cout_pad, K]
+        (K = taps x channels, channels fastest) with zero rows beyond Cout.  A fused 1x1 shortcut
+        ``ext = (e1, e2, w_sc, b_sc)`` is appended along K: its input becomes a second A source
+        (centre tap) and its bias joins the conv bias."""
+        Cout = w.shape[0]
+        wt = w.permute(0, 2, 3, 1).reshape(Cout, -1)
+        if ext is not None:
+            e1, e2, we, be = ext
+            wt = torch.cat([wt, we.detach().to(self.dev, torch.float32).reshape(Cout, -1)], 1)
+            op.inp[8] = e1.data_ptr()
+            op.inp[9] = e2.data_ptr() if e2 is not None else None
+            op.i[L.CONV_EXT_C1] = e1.shape[-1]
+            op.i[L.CONV_EXT_C2] = e2.shape[-1] if e2 is not None else 0
+            if be is not None:
+                b32 = self._w((b32 if b32 is not None else 0) + be.detach().to(self.dev, torch.float32))
+        if cout_pad != Cout:
+            wt = torch.cat([wt, wt.new_zeros(cout_pad - Cout, wt.shape[1])], 0)
+            if b32 is not None:
+                b32 = self._w(torch.cat([b32, b32.new_zeros(cout_pad - Cout)]))
+        op.i[L.CONV_COUT] = cout_pad
+        op.inp[4] = self._w_bf16(wt).data_ptr()
+        op.inp[5] = b32.data_ptr() if b32 is not None else None
 
     def _op(self, kind, engine=L.ENGINE_SIMT):
         op = L.Op()
@@ -295,39 +320,16 @@ class Plan:
         w = w_oihw.detach().to(self.dev, torch.float32)
         done = False
         if affine is not None:
-            # GroupNorm(+SiLU) applied on load inside the tensor-core kernel
+            # GroupNorm(+SiLU) applied on load inside the tensor-core kernel; the network head's
+            # zero rows fill a 64-wide N tile
             op.engine = L.ENGINE_TC_GN
             op.inp[6] = affine.data_ptr()
             i[L.CONV_GN_SILU] = int(gn_silu)
-            wt = w.permute(0, 2, 3, 1).reshape(Cout, -1)
-            if ext is not None:      # 1x1 shortcut over the (un-normalised) block input: extra K-blocks
-                e1, e2, we, be = ext
-                wt = torch.cat([wt, we.detach().to(self.dev, torch.float32).reshape(Cout, -1)], 1)
-                op.inp[8] = e1.data_ptr()
-                op.inp[9] = e2.data_ptr() if e2 is not None else None
-                i[L.CONV_EXT_C1] = e1.shape[-1]
-                i[L.CONV_EXT_C2] = e2.shape[-1] if e2 is not None else 0
-                if be is not None:
-                    b32 = self._w((bias.detach().to(self.dev, torch.float32) if bias is not None else 0) +
-                                  be.detach().to(self.dev, torch.float32))
-                    op.inp[5] = b32.data_ptr()
-            if out_nchw_f32 and Cout % 64:          # network head: zero rows up to a 64-wide N tile
-                cpad = -(-Cout // 64) * 64
-                wt = torch.cat([wt, wt.new_zeros(cpad - Cout, wt.shape[1])], 0)
-                if b32 is not None:
-                    b32 = self._w(torch.cat([b32, b32.new_zeros(cpad - Cout)]))
-                    op.inp[5] = b32.data_ptr()
-                i[L.CONV_COUT] = cpad
+            self._pack_tc_conv(op, w, b32, ext, -(-Cout // 64) * 64 if out_nchw_f32 else Cout)
+            if out_nchw_f32:
                 op.f[1] = float(Cout)
-            elif out_nchw_f32:
-                op.f[1] = float(Cout)
-            if self.x3:      # weight planes [2][Cout, K]
-                hi = wt.to(torch.bfloat16)
-                wt = torch.cat([hi, (wt - hi.to(torch.float32)).to(torch.bfloat16)], 0)
-            wt = self._w(wt, torch.bfloat16)
-            op.inp[4] = wt.data_ptr()
             mg = None
-            if self.fused_stats and want_stats and not out_nchw_f32 and (OH * OW) % 32 == 0:
+            if want_stats and not out_nchw_f32 and (OH * OW) % 32 == 0:
                 mg = self._mg_buffer(N, Cout)
                 op.out[1] = mg.data_ptr()
             if not self.dry:
@@ -338,38 +340,11 @@ class Plan:
             done = True
         elif self.tc and allow_tc and not in_nchw:
             op.engine = L.ENGINE_TC
-            cout_pad = Cout
-            if out_nchw_f32 and Cout % 32:
-                cout_pad = -(-Cout // 32) * 32       # zero rows; the epilogue writes Cout planes
-            wt = w.permute(0, 2, 3, 1).reshape(Cout, -1)
-            if ext is not None:
-                # fused 1x1 shortcut: its weight is appended along K, its input becomes a second
-                # A source (centre tap), its bias joins the conv bias
-                e1, e2, we, be = ext
-                wt = torch.cat([wt, we.detach().to(self.dev, torch.float32).reshape(Cout, -1)], 1)
-                op.inp[8] = e1.data_ptr()
-                op.inp[9] = e2.data_ptr() if e2 is not None else None
-                i[L.CONV_EXT_C1] = e1.shape[-1]
-                i[L.CONV_EXT_C2] = e2.shape[-1] if e2 is not None else 0
-                if be is not None:
-                    b32 = self._w((bias.detach().to(self.dev, torch.float32) if bias is not None else 0) +
-                                  be.detach().to(self.dev, torch.float32))
-                    op.inp[5] = b32.data_ptr()
-            if cout_pad != Cout:
-                wt = torch.cat([wt, wt.new_zeros(cout_pad - Cout, wt.shape[1])], 0)
-                if b32 is not None:
-                    b32 = self._w(torch.cat([b32, b32.new_zeros(cout_pad - Cout)]))
-                    op.inp[5] = b32.data_ptr()
-            if self.x3:      # weight planes [2][Cout, K]: hi = rn(w), lo = rn(w - hi)
-                hi = wt.to(torch.bfloat16)
-                wt = torch.cat([hi, (wt - hi.to(torch.float32)).to(torch.bfloat16)], 0)
-            wt = self._w(wt, torch.bfloat16)
-            op.inp[4] = wt.data_ptr()
-            i[L.CONV_COUT] = cout_pad
-            op.i[L.CONV_OUT_DTYPE] = L.F32 if out_nchw_f32 else self.acode
+            # NCHW head: zero rows up to a 32-wide N tile, the epilogue writes Cout planes
+            self._pack_tc_conv(op, w, b32, ext, -(-Cout // 32) * 32 if out_nchw_f32 else Cout)
             op.f[1] = float(Cout)                    # valid output channels (NCHW f32 epilogue)
             mg = None
-            if self.fused_stats and want_stats and not out_nchw_f32 and (OH * OW) % 32 == 0 and Cout % 32 == 0:
+            if want_stats and not out_nchw_f32 and (OH * OW) % 32 == 0 and Cout % 32 == 0:
                 mg = self._mg_buffer(N, Cout)
                 op.out[1] = mg.data_ptr()
             rc = self._tc_eligible(op) if self.dry else self.lib.psld_op_prepare(C.byref(op))
@@ -424,20 +399,16 @@ class Plan:
         op.inp[0] = qkv.data_ptr()
         fusable = Cc % 64 == 0 and 64 <= Cc <= 256 and HW in (128, 256)
         if proj is not None:
-            if not (self.tc and fusable) or os.environ.get("PSLD_ATTN_FUSE_PROJ", "1") == "0":
+            if not (self.tc and fusable):
                 return None
             w3, b3, x, scale, o = proj
             op.i[L.ATTN_PROJ] = 1
             op.f[1] = float(scale)
-            w3 = w3.detach().to(self.dev, torch.float32)
-            if self.x3:          # weight planes [2][C out, C in]
-                hi = w3.to(torch.bfloat16)
-                w3 = torch.cat([hi, (w3 - hi.to(torch.float32)).to(torch.bfloat16)], 0)
-            op.inp[1] = self._w(w3, torch.bfloat16).data_ptr()
+            op.inp[1] = self._w_bf16(w3.detach().to(self.dev, torch.float32)).data_ptr()
             op.inp[2] = self._w(b3).data_ptr() if b3 is not None else None
             op.inp[3] = x.data_ptr()
             mg = None
-            if self.fused_stats and Cc % 32 == 0:
+            if Cc % 32 == 0:
                 mg = self._mg_buffer(self.B, Cc)
                 op.out[1] = mg.data_ptr()
         else:
@@ -512,17 +483,14 @@ class Plan:
         (layerspp.py:264-274).  ``h`` is consumed."""
         N, H, W, _ = h.shape
         has_sc = hasattr(m, "Conv_2")
-        gn1 = self.fuse_gn_residual or os.environ.get("PSLD_TC_FUSE_GN1", "1") == "1"
-        if gn1 and has_sc:
-            # blocks with a Conv_2 shortcut.  bf16: they keep the unfused Conv_1 (apply pass +
-            # conv_tc with the shortcut as K-extension): the fused kernel accepts the extension
-            # too, but its two big operand buffers cannot hide the load latency of one-tap chunks
-            # (measured +1.1 ms of conv for -0.64 ms of GroupNorm per step).  bf16x3: the fused
-            # kernel streams the shortcut tiles through a 3-slot ring of their own, so the
-            # extension costs what it costs in conv_tc and the apply pass goes away.
-            # PSLD_TC_FUSE_GN_EXT overrides either default.
-            gn1 = (os.environ.get("PSLD_TC_FUSE_GN_EXT", "1" if self.x3 else "0") == "1"
-                   and self._ext_fusable(h, x1, x2, m.out_ch))
+        # GroupNorm_1 is applied on load inside Conv_1 of identity-shortcut blocks.  Blocks with a
+        # Conv_2 shortcut: bf16 keeps the unfused Conv_1 (apply pass + conv_tc with the shortcut as
+        # K-extension): the fused kernel accepts the extension too, but its two big operand buffers
+        # cannot hide the load latency of one-tap chunks (measured +1.1 ms of conv for -0.64 ms of
+        # GroupNorm per step).  bf16x3: the fused kernel streams the shortcut tiles through a
+        # 3-slot ring of their own, so the extension costs what it costs in conv_tc and the apply
+        # pass goes away.
+        gn1 = not has_sc or (self.x3 and self._ext_fusable(h, x1, x2, m.out_ch))
         if gn1 and self._gn_fusable(h, None, m.out_ch):
             aff1 = self.op_gn(h, None, m.GroupNorm_1, True, H * W, affine_only=True)
             b, b_aff = h, aff1
@@ -667,7 +635,7 @@ class Plan:
                 m = mods[i]; i += 1
                 h = self.resblock(m, h, None, offs[id(m)])
         assert not hs
-        if self._gn_fusable(h, None, 64) and os.environ.get("PSLD_TC_FUSE_GN_HEAD", "1") == "1":
+        if self._gn_fusable(h, None, 64):
             # final act(GroupNorm(h)) -> conv3x3 -> fp32 NCHW eps as one GroupNorm-on-load conv
             aff = self.op_gn(h, None, mods[i], True, h.shape[1] * h.shape[2], affine_only=True); i += 1
             self.eps = self.op_conv(h, None, mods[i].weight, mods[i].bias, ks=3, out_nchw_f32=True,

@@ -8,8 +8,6 @@ Tolerances (stated, per kernel):
 """
 import ctypes as C
 
-import os
-
 import numpy as np
 import pytest
 import torch
@@ -424,8 +422,6 @@ def test_conv_tc_stride2(case):
 def test_conv_gn_fused(case, silu):
     """GroupNorm(+SiLU)-on-load 3x3 conv (PSLD_ENGINE_TC_GN): per-(sample, channel) affine + SiLU
     applied to the raw tile in shared memory, three shifted operand variants, 2-CTA MMA."""
-    if os.environ.get("PSLD_TC_FUSE_GN", "1") == "0":
-        pytest.skip("fused GroupNorm conv disabled by PSLD_TC_FUSE_GN=0")
     N, H, W, C1, C2, Cout = case
     r = _rng(sum(case) + 5)
     x1 = _t(r.standard_normal((N, H, W, C1)) * 1.7 + 0.3, torch.bfloat16)
@@ -479,8 +475,6 @@ def test_conv_tc_fused_shortcut(case):
 def test_conv_gn_fused_with_shortcut(case):
     """GroupNorm_1+SiLU on load -> Conv_1, plus the Conv_2 1x1 shortcut over the RAW block input
     cat(e1, e2) as extra K-blocks of the same accumulation (layerspp.py:262-274)."""
-    if os.environ.get("PSLD_TC_FUSE_GN", "1") == "0":
-        pytest.skip("fused GroupNorm conv disabled by PSLD_TC_FUSE_GN=0")
     N, H, W, Cb, E1, E2, Cout = case
     r = _rng(sum(case) + 13)
     h = _t(r.standard_normal((N, H, W, Cb)) * 1.5 + 0.2, torch.bfloat16)
@@ -506,8 +500,6 @@ def test_conv_gn_fused_with_shortcut(case):
 def test_conv_gn_fused_output_head():
     """Final act(GroupNorm(h)) -> conv3x3 -> 6 channels as fp32 NCHW through the GroupNorm-on-load
     kernel (Cout zero-padded to one 64-wide N tile)."""
-    if os.environ.get("PSLD_TC_FUSE_GN", "1") == "0":
-        pytest.skip("fused GroupNorm conv disabled by PSLD_TC_FUSE_GN=0")
     r = _rng(78)
     N, H, W, Cin = 3, 32, 32, 128
     x = _t(r.standard_normal((N, H, W, Cin)) * 1.3 + 0.1, torch.bfloat16)
