@@ -239,6 +239,13 @@ def rel_l2(a, b):
     return float((a - b).norm() / b.norm().clamp_min(1e-300))
 
 
+def per_sample_rel_l2(a, b):
+    """rel-L2 of every sample (leading dimension) separately, as a float64 tensor."""
+    a, b = val(a).double(), val(b).double().to(val(a).device)
+    d = (a - b).reshape(a.shape[0], -1).norm(dim=1)
+    return (d / b.reshape(b.shape[0], -1).norm(dim=1).clamp_min(1e-300)).cpu()
+
+
 def max_rel(a, b):
     a, b = val(a).double().cpu(), val(b).double().cpu()
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-300))
