@@ -321,6 +321,11 @@ enum { PSLD_FIR_N = 0, PSLD_FIR_H, PSLD_FIR_W, PSLD_FIR_C, PSLD_FIR_UP, PSLD_FIR
  *            zeroes it before the launch (PSLD_OP_ZERO) (TC engines, bf16 NHWC output,
  *            OH*OW % 32 == 0), or NULL
  *   weight layout: SIMT engine f32 [K, Cout] ; TC engine bf16 [Cout, K], K = (ky*KW+kx)*Cin + c
+ *   OUT_LAYOUT = NCHW (the network's output head): y is fp32 [N, V, OH, OW] with V = Cout (SIMT) or
+ *           V = f[1] valid channels of a zero-padded Cout (TC engines); the residual, if any, is then
+ *           fp32 NCHW of the same shape (RES_DTYPE = PSLD_F32) and is added to those V channels
+ *           (progressive=output_skip: the upsampled output pyramid, ncsnpp.py:414-418)
+ *   PSLD_ENGINE_TC output widths: OW a power of two in 4..128, or 256 for stride 1 (half-row tiles)
  *   i: N, H, W, C1, C2, COUT, KS (1|3), STRIDE, PAD, OH, OW, IN_LAYOUT, OUT_LAYOUT,
  *      IN_DTYPE, OUT_DTYPE, RES_DTYPE, TEMB_OFF, TEMB_BSTRIDE ; f[0] = scale            */
 enum { PSLD_CONV_N = 0, PSLD_CONV_H, PSLD_CONV_W, PSLD_CONV_C1, PSLD_CONV_C2, PSLD_CONV_COUT,

@@ -838,12 +838,14 @@ int prepare_conv_gn_tc(psld_op& op) {
   const int cm = x3 ? 2 : 1;
   if (op.i[PSLD_CONV_IN_LAYOUT] != PSLD_NHWC || (!head && op.i[PSLD_CONV_OUT_LAYOUT] != PSLD_NHWC))
     return unsupported("NHWC only");
-  if (head && (op.out[1] || op.in[2])) return unsupported("head: no statistics / residual");
+  if (head && op.out[1]) return unsupported("head: no statistics");
+  if (head && op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != PSLD_F32)
+    return unsupported("head residual must be fp32 NCHW");
   if (KS != 3 || op.i[PSLD_CONV_STRIDE] != 1 || op.i[PSLD_CONV_PAD] != 1) return unsupported("3x3 s1 p1 only");
   if (C1 % TC_BLOCK_K || C2 % TC_BLOCK_K) return unsupported("Cin %% 64 != 0");
   if (Cout % 64 || Cout > 256 && Cout % 256) return unsupported("Cout");
   if (!((W == 32 && H >= 4) || (W == 16 && H >= 8)) || (H & (H - 1))) return unsupported("map must be 16x16+ / 32x32+ wide tiles");
-  if (op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != adt) return unsupported("residual dtype");
+  if (!head && op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != adt) return unsupported("residual dtype");
   if (!op.in[0] || !op.in[4] || !op.in[6] || !op.out[0] || (C2 > 0 && !op.in[1])) {
     set_error("conv_gn_tc: null pointer");
     return PSLD_EINVAL;

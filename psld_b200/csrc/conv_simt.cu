@@ -128,7 +128,12 @@ conv_simt_kernel(const ConvP p) {
       if (co < p.Cout) {
         if (p.bias) v += p.bias[co];
         if (p.temb) v += p.temb[(int64_t)n * p.temb_bstride + p.temb_off + co];
-        if (p.res) v += ld_elt<TO>((const TO*)p.res + m * (p.Cout * Elt<TO>::kMul) + co, p.Cout);
+        if (p.res) {
+          if (p.out_layout == PSLD_NCHW)     // fp32 NCHW residual of the NCHW head
+            v += ((const float*)p.res)[(((int64_t)n * p.Cout + co) * p.OH + oy) * p.OW + ox];
+          else
+            v += ld_elt<TO>((const TO*)p.res + m * (p.Cout * Elt<TO>::kMul) + co, p.Cout);
+        }
         v *= p.scale;
       }
       o[j] = v;
@@ -174,8 +179,7 @@ int run_conv_simt(const psld_op& op, cudaStream_t s) {
                  p.OW == (p.W + 2 * p.pad - p.KS) / p.stride + 1, "conv: OH/OW mismatch");
   PSLD_CHECK_ARG(p.in_layout == PSLD_NHWC || (idt == PSLD_F32 && p.C2 == 0),
                  "conv: NCHW input must be fp32 single-source");
-  PSLD_CHECK_ARG(p.out_layout == PSLD_NHWC || (odt == PSLD_F32 && !p.res),
-                 "conv: NCHW output must be fp32 without residual");
+  PSLD_CHECK_ARG(p.out_layout == PSLD_NHWC || odt == PSLD_F32, "conv: NCHW output must be fp32");
   PSLD_CHECK_ARG(!p.res || op.i[PSLD_CONV_RES_DTYPE] == odt, "conv: residual dtype != out dtype");
   const int64_t M = (int64_t)p.N * p.OH * p.OW;
   dim3 grid((unsigned)ceil_div(M, BM), (unsigned)ceil_div(p.Cout, BN));

@@ -155,7 +155,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
         const int n_tile = unit % p.n_tiles_n;
         const int m_tile = kPair ? 2 * (unit / p.n_tiles_n) + (int)rank : unit / p.n_tiles_n;
         const int n0 = (m_tile / p.tiles_y) * p.BN_img;
-        const int y0 = (m_tile % p.tiles_y) * p.BH * p.stride - p.pad;
+        const int t_img = m_tile % p.tiles_y;                      // (row group, x-tile) in the image
+        const int y0 = (t_img / p.tiles_x) * p.BH * p.stride - p.pad;
+        const int x0 = (t_img % p.tiles_x) * TC_BLOCK_M;           // 256-wide rows: two 128-pixel halves
         const int b_rows = kPair ? (bn >> 1) : bn;                 // weight rows this CTA loads
         const CUtensorMap* tmW = nsub < 0 ? &tmB : &tmB2;
         const int bn0 = n_tile * p.block_n + (nsub < 0 ? 0 : nsub * bn) + (kPair ? (int)rank * b_rows : 0);
@@ -172,9 +174,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
                   const bool s1 = cc < p.kchunks1;
                   const CUtensorMap* tmA = s1 ? &tmA1 : &tmA2;
                   const int c0 = (s1 ? cc : cc - p.kchunks1) * TC_BLOCK_K;
-                  load_a(sa, tmA, full_bar(stage), c0, kx - p.pad, y0 + ky, n0);
+                  load_a(sa, tmA, full_bar(stage), c0, x0 + kx - p.pad, y0 + ky, n0);
                   if (kX3)
-                    load_a(sa + TC_A_BYTES, tmA, full_bar(stage), c0 + (s1 ? p.lo1 : p.lo2), kx - p.pad,
+                    load_a(sa + TC_A_BYTES, tmA, full_bar(stage), c0 + (s1 ? p.lo1 : p.lo2), x0 + kx - p.pad,
                            y0 + ky, n0);
                 } else {
                   load_b(sa + Cfg::kBOff, tmW, full_bar(stage), kb * TC_BLOCK_K, bn0);
@@ -197,9 +199,9 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
               const bool s1 = cc < p.ext_kchunks1;
               const CUtensorMap* tmE = s1 ? &tmE1 : &tmE2;
               const int c0 = (s1 ? cc : cc - p.ext_kchunks1) * TC_BLOCK_K;
-              load_a(sa, tmE, full_bar(stage), c0, 0, y0 + p.pad, n0);
+              load_a(sa, tmE, full_bar(stage), c0, x0, y0 + p.pad, n0);
               if (kX3)
-                load_a(sa + TC_A_BYTES, tmE, full_bar(stage), c0 + (s1 ? p.loe1 : p.loe2), 0,
+                load_a(sa + TC_A_BYTES, tmE, full_bar(stage), c0 + (s1 ? p.loe1 : p.loe2), x0,
                        y0 + p.pad, n0);
             } else {
               load_b(sa + Cfg::kBOff, tmW, full_bar(stage), kb * TC_BLOCK_K, bn0);
@@ -323,14 +325,14 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA1, const __grid_constant__
 }
 
 // ---------------------------------------------------------------- host side
-// Activation map over the INPUT tensor [N, H, W, C]; the box covers OW x BH x BN output positions
+// Activation map over the INPUT tensor [N, H, W, C]; the box covers BW x BH x BN output positions
 // visited with element stride `stride` (TMA loads ceil(box / stride) elements per dimension).
 // (split bf16: C = 2 x channels, the row holds [hi | lo])
-static int encode_act_map(CUtensorMap* tm, const void* ptr, int N, int H, int W, int C, int OW,
+static int encode_act_map(CUtensorMap* tm, const void* ptr, int N, int H, int W, int C, int BW,
                           int BH, int BN_img, int stride) {
   const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)N};
   const cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)W * C * 2, (cuuint64_t)H * W * C * 2};
-  const cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)(OW * stride), (cuuint32_t)(BH * stride),
+  const cuuint32_t box[4] = {(cuuint32_t)TC_BLOCK_K, (cuuint32_t)(BW * stride), (cuuint32_t)(BH * stride),
                              (cuuint32_t)BN_img};
   const cuuint32_t estr[4] = {1, (cuuint32_t)stride, (cuuint32_t)stride, 1};
   return encode_bf16_map(tm, ptr, 4, dims, strides, box, estr, "activation");
@@ -355,8 +357,10 @@ int prepare_conv_tc(psld_op& op) {
   if (op.i[PSLD_CONV_OUT_DTYPE] != (head ? PSLD_F32 : adt))
     return unsupported("output must be NHWC of the input's element type, or fp32 NCHW");
   if (op.i[PSLD_CONV_IN_LAYOUT] != PSLD_NHWC) return unsupported("input layout must be NHWC");
-  if (head && (op.in[2] || op.f[1] < 1.0f || (int)op.f[1] > Cout))
-    return unsupported("NCHW head takes no residual and needs f[1] = valid channels");
+  if (head && (op.f[1] < 1.0f || (int)op.f[1] > Cout))
+    return unsupported("NCHW head needs f[1] = valid channels");
+  if (head && op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != PSLD_F32)
+    return unsupported("NCHW head residual must be fp32 NCHW");
   const int stride = op.i[PSLD_CONV_STRIDE], pad = op.i[PSLD_CONV_PAD];
   const bool same = stride == 1 && pad == KS / 2 && (KS == 1 || KS == 3);
   const bool down2 = stride == 2 && pad == 0 && KS == 3 && C2 == 0;   // conv_downsample_2d's conv
@@ -368,10 +372,9 @@ int prepare_conv_tc(psld_op& op) {
   }
   if (C1 % TC_BLOCK_K || C2 % TC_BLOCK_K) return unsupported("Cin %% 64 != 0");
   if (Cout % 32) return unsupported("Cout %% 32 != 0");
-  if (!is_pow2(OW) || !is_pow2(OH) || OW > 128 || OW < 4)
-    return unsupported("output W,H must be pow2, 4..128");
-  if (stride == 2 && OW * stride > 256) return unsupported("stride-2 box too wide");
-  if (op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != adt) return unsupported("residual dtype");
+  if (!is_pow2(OW) || !is_pow2(OH) || OW > (same ? 256 : 128) || OW < 4)
+    return unsupported("output W,H must be pow2, 4..256 (stride 1) or 4..128");
+  if (!head && op.in[2] && op.i[PSLD_CONV_RES_DTYPE] != adt) return unsupported("residual dtype");
   if (x3 && !head && (OH * OW) % 32) return unsupported("split bf16 output needs H*W %% 32 == 0");
   if (!op.in[0] || !op.in[4] || !op.out[0] || (C2 > 0 && !op.in[1])) {
     set_error("conv_tc: null pointer");
@@ -383,21 +386,23 @@ int prepare_conv_tc(psld_op& op) {
   int block_n = 0;
   for (int cand : {256, 128, 64, 32})
     if (Cout % cand == 0) { block_n = cand; break; }
-  int BH = 128 / OW;
+  // M tile = 128 output pixels: whole rows of BN_img images, or half a row when OW = 256
+  const int BW = OW < TC_BLOCK_M ? OW : TC_BLOCK_M;
+  int BH = 128 / BW;
   if (BH > OH) BH = OH;
-  const int BN_img = 128 / (OW * BH);
+  const int BN_img = 128 / (BW * BH);
   if (BN_img > 256) return unsupported("image too small");
 
   const int sms = sm_count();
   // 2-CTA pairs whenever there are at least two M tiles
-  const int64_t m_tiles_all = (int64_t)((N + BN_img - 1) / BN_img) * (OH / BH);
+  const int64_t m_tiles_all = (int64_t)((N + BN_img - 1) / BN_img) * (OH / BH) * (OW / BW);
   const bool pair = m_tiles_all >= 2 && sms >= 2;
   ConvTcState* st = new (std::nothrow) ConvTcState();
   if (!st) { set_error("conv_tc: out of host memory"); return PSLD_ECUDA; }
-  int rc = encode_act_map(&st->a1, op.in[0], N, H, W, cm * C1, OW, BH, BN_img, stride);
+  int rc = encode_act_map(&st->a1, op.in[0], N, H, W, cm * C1, BW, BH, BN_img, stride);
   if (rc == PSLD_OK)
-    rc = C2 > 0 ? encode_act_map(&st->a2, op.in[1], N, H, W, cm * C2, OW, BH, BN_img, stride)
-                : encode_act_map(&st->a2, op.in[0], N, H, W, cm * C1, OW, BH, BN_img, stride);
+    rc = C2 > 0 ? encode_act_map(&st->a2, op.in[1], N, H, W, cm * C2, BW, BH, BN_img, stride)
+                : encode_act_map(&st->a2, op.in[0], N, H, W, cm * C1, BW, BH, BN_img, stride);
   const int E1 = op.i[PSLD_CONV_EXT_C1], E2 = op.i[PSLD_CONV_EXT_C2];
   const bool ext = op.in[8] != nullptr && E1 > 0;
   if (ext && (stride != 1 || E1 % TC_BLOCK_K || E2 % TC_BLOCK_K || (E2 > 0 && !op.in[9]))) {
@@ -405,11 +410,11 @@ int prepare_conv_tc(psld_op& op) {
     return unsupported("1x1 extension needs stride 1 and channel counts %% 64 == 0");
   }
   if (rc == PSLD_OK)
-    rc = ext ? encode_act_map(&st->e1, op.in[8], N, OH, OW, cm * E1, OW, BH, BN_img, 1)
-             : encode_act_map(&st->e1, op.in[0], N, H, W, cm * C1, OW, BH, BN_img, stride);
+    rc = ext ? encode_act_map(&st->e1, op.in[8], N, OH, OW, cm * E1, BW, BH, BN_img, 1)
+             : encode_act_map(&st->e1, op.in[0], N, H, W, cm * C1, BW, BH, BN_img, stride);
   if (rc == PSLD_OK)
-    rc = (ext && E2 > 0) ? encode_act_map(&st->e2, op.in[9], N, OH, OW, cm * E2, OW, BH, BN_img, 1)
-                         : encode_act_map(&st->e2, op.in[0], N, H, W, cm * C1, OW, BH, BN_img, stride);
+    rc = (ext && E2 > 0) ? encode_act_map(&st->e2, op.in[9], N, OH, OW, cm * E2, BW, BH, BN_img, 1)
+                         : encode_act_map(&st->e2, op.in[0], N, H, W, cm * C1, BW, BH, BN_img, stride);
   const int K = KS * KS * (C1 + C2) + (ext ? E1 + E2 : 0);
   // split bf16 weights: two planes [2][Cout, K] seen as one [2*Cout, K] matrix
   if (rc == PSLD_OK) rc = encode_w_map(&st->b, op.in[4], cm * Cout, K, pair ? block_n / 2 : block_n);

@@ -24,16 +24,18 @@ struct ConvTcParams {
   const __nv_bfloat16* res;
   __nv_bfloat16* y;
   float* y_nchw;             // when non-null: fp32 NCHW output, first cout_valid channels only
-  double* mg_stats;          // optional [N, Cout/4, 2] per-sample (sum, sumsq) of the output per 4
+  const float* res_nchw;     // optional fp32 NCHW residual of the y_nchw head (same shape as y_nchw)
+  double* mg_stats;         // optional [N, Cout/4, 2] per-sample (sum, sumsq) of the output per 4
                              // channels, accumulated with atomics (zeroed by the caller)
   int cout_valid;
   float scale;
   int temb_off, temb_bstride;
   int H, W, HW, Cout;        // OUTPUT map size (== input size for the stride-1 'same' case)
   int stride, pad;           // 1/KS/2, or 2/0 (3x3 stride-2 conv on a pre-padded input)
-  int BH, BN_img;            // output rows / images per tile: W*BH*BN_img == 128; the TMA box is
-                             // {64, W*stride, BH*stride, BN_img} traversed with element stride
-  int tiles_y;               // H / BH
+  int BH, BN_img;            // output rows / images per tile: min(W,128)*BH*BN_img == 128; the TMA box
+                             // is {64, min(W,128)*stride, BH*stride, BN_img} traversed with element stride
+  int tiles_x;               // tiles per output row: W / 128 for W = 256 (BH = BN_img = 1), else 1
+  int tiles_y;               // M tiles per BN_img images: (H / BH) * tiles_x
   int kchunks1, kchunks;     // 64-channel chunks in source 1 / in total (C1+C2)/64
   int taps, KS;
   int ext_kchunks1, ext_kchunks;   // 64-channel chunks of the fused 1x1 shortcut input (0 = none)
@@ -518,13 +520,22 @@ __device__ __forceinline__ void tc_epilogue_tile(const ConvTcParams& p, uint32_t
 #pragma unroll
       for (int j = 0; j < 32; ++j) v[j] *= p.scale;
       if (p.y_nchw) {
-        // network output head (ncsnpp.py:430): fp32 NCHW, lanes = consecutive pixels
+        // network output head (ncsnpp.py:430): fp32 NCHW, lanes = consecutive pixels; the output
+        // pyramid of progressive=output_skip arrives as an fp32 NCHW residual (ncsnpp.py:414-418)
         const int64_t pix = m - (int64_t)img * p.HW;
+        if (p.res_nchw) {
 #pragma unroll
-        for (int j = 0; j < 32; ++j) {
-          const int co = co0 + j;
-          if (co < p.cout_valid)
-            p.y_nchw[((int64_t)img * p.cout_valid + co) * p.HW + pix] = v[j];
+          for (int j = 0; j < 32; ++j) {
+            const int64_t o = ((int64_t)img * p.cout_valid + co0 + j) * p.HW + pix;
+            if (co0 + j < p.cout_valid) p.y_nchw[o] = fmaf(p.scale, __ldg(p.res_nchw + o), v[j]);
+          }
+        } else {
+#pragma unroll
+          for (int j = 0; j < 32; ++j) {
+            const int co = co0 + j;
+            if (co < p.cout_valid)
+              p.y_nchw[((int64_t)img * p.cout_valid + co) * p.HW + pix] = v[j];
+          }
         }
       } else {
 #pragma unroll
@@ -610,9 +621,10 @@ static inline void tc_conv_params(ConvTcParams& p, const psld_op& op, bool head,
   const bool ext = op.in[8] != nullptr && E1 > 0;
   p.bias = (const float*)op.in[5];
   p.temb = (const float*)op.in[3];
-  p.res = (const __nv_bfloat16*)op.in[2];
+  p.res = head ? nullptr : (const __nv_bfloat16*)op.in[2];
   p.y = head ? nullptr : (__nv_bfloat16*)op.out[0];
   p.y_nchw = head ? (float*)op.out[0] : nullptr;
+  p.res_nchw = head ? (const float*)op.in[2] : nullptr;
   p.cout_valid = head ? (int)op.f[1] : Cout;
   p.mg_stats = (double*)op.out[1];
   p.scale = op.f[0];
@@ -620,7 +632,9 @@ static inline void tc_conv_params(ConvTcParams& p, const psld_op& op, bool head,
   p.temb_bstride = op.i[PSLD_CONV_TEMB_BSTRIDE];
   p.H = OH; p.W = OW; p.HW = OH * OW; p.Cout = Cout;
   p.stride = op.i[PSLD_CONV_STRIDE]; p.pad = op.i[PSLD_CONV_PAD];
-  p.BH = BH; p.BN_img = BN_img; p.tiles_y = OH / BH;
+  p.BH = BH; p.BN_img = BN_img;
+  p.tiles_x = OW > TC_BLOCK_M ? OW / TC_BLOCK_M : 1;
+  p.tiles_y = OH / BH * p.tiles_x;
   p.kchunks1 = C1 / TC_BLOCK_K; p.kchunks = (C1 + C2) / TC_BLOCK_K;
   p.taps = KS * KS; p.KS = KS;
   p.ext_kchunks1 = ext ? E1 / TC_BLOCK_K : 0;

@@ -12,9 +12,11 @@ is compiled once per (batch, #time rows) into a flat "program" of ``psld_op`` re
 and replayed by the native executor ``psld_program_run`` — there is no per-layer Python or
 PyTorch dispatch on the hot path and no eager fallback.
 
-Supported configuration space (what the BASELINE configs and the shipped sampling scripts
-use): ``resblock_type=biggan``, ``progressive=none``, ``progressive_input in {none,residual}``,
-``embedding_type in {fourier,positional}``, ``fir in {True,False}``, ``nonlinearity=swish``.
+Supported configuration space (the BASELINE configs, the shipped sampling scripts and the
+high-resolution NCSN++ configurations of the score-SDE family): ``resblock_type=biggan``,
+``progressive in {none,output_skip}``, ``progressive_input in {none,residual,input_skip}``,
+``progressive_combine=sum``, ``embedding_type in {fourier,positional}``, ``fir in {True,False}``
+(``progressive_input=residual`` needs ``fir=True``), ``nonlinearity=swish``.
 """
 from __future__ import annotations
 
@@ -134,6 +136,15 @@ class PyramidDownsample(nn.Module):
         self.in_ch, self.out_ch = in_ch, out_ch
 
 
+class Combine(nn.Module):
+    """Merges the input pyramid into the down path: ``Conv_0(pyr) + h`` (reference layerspp.py:
+    Combine with ``method='sum'``; ``Conv_0`` = ddpm_conv1x1)."""
+
+    def __init__(self, dim1, dim2):
+        super().__init__()
+        self.Conv_0 = _conv(dim1, dim2, 1)
+
+
 # ----------------------------------------------------------------------------------------
 # The network
 # ----------------------------------------------------------------------------------------
@@ -149,11 +160,17 @@ class NCSNpp(nn.Module):
             raise NotImplementedError("psld_b200 NCSNpp: only nonlinearity=swish (SiLU)")
         if str(sf.resblock_type).lower() != "biggan":
             raise NotImplementedError("psld_b200 NCSNpp: only resblock_type=biggan")
-        if str(sf.progressive).lower() != "none":
-            raise NotImplementedError("psld_b200 NCSNpp: only progressive=none")
+        self.progressive = str(sf.progressive).lower()
+        if self.progressive not in ("none", "output_skip"):
+            raise NotImplementedError("psld_b200 NCSNpp: progressive must be none|output_skip")
         self.progressive_input = str(sf.progressive_input).lower()
-        if self.progressive_input not in ("none", "residual"):
-            raise NotImplementedError("psld_b200 NCSNpp: progressive_input must be none|residual")
+        if self.progressive_input not in ("none", "residual", "input_skip"):
+            raise NotImplementedError("psld_b200 NCSNpp: progressive_input must be none|residual|input_skip")
+        combine = str(getattr(sf, "progressive_combine", "sum")).lower()
+        if self.progressive_input == "input_skip" and combine != "sum":
+            # cat would widen every skip tensor by the pyramid's channels: convolutions writing into a
+            # channel slice of a wider buffer, which no known configuration needs
+            raise NotImplementedError("psld_b200 NCSNpp: input_skip needs progressive_combine=sum")
         self.embedding_type = str(sf.embedding_type).lower()
         assert self.embedding_type in ["fourier", "positional"]
         self.nf = nf = int(sf.nf)
@@ -208,7 +225,9 @@ class NCSNpp(nn.Module):
                 hs_c.append(in_ch)
             if lvl != self.num_resolutions - 1:
                 mods.append(RB(in_ch=in_ch, down=True))
-                if self.progressive_input == "residual":
+                if self.progressive_input == "input_skip":
+                    mods.append(Combine(pyr_ch, in_ch))       # pyr_ch stays in_ch of the network
+                elif self.progressive_input == "residual":
                     mods.append(PyramidDownsample(pyr_ch, in_ch))
                     pyr_ch = in_ch
                 hs_c.append(in_ch)
@@ -223,11 +242,15 @@ class NCSNpp(nn.Module):
                 in_ch = out_ch
             if self.all_resolutions[lvl] in self.attn_resolutions:
                 mods.append(AttnBlockpp(in_ch, init_scale))
+            if self.progressive == "output_skip":      # this level's output head
+                mods.append(_gn(in_ch))
+                mods.append(_conv(in_ch, self.out_ch, 3, init_scale))
             if lvl != 0:
                 mods.append(RB(in_ch=in_ch, up=True))
         assert not hs_c
-        mods.append(_gn(in_ch))
-        mods.append(_conv(in_ch, self.out_ch, 3, init_scale))
+        if self.progressive != "output_skip":
+            mods.append(_gn(in_ch))
+            mods.append(_conv(in_ch, self.out_ch, 3, init_scale))
         self.all_modules = nn.ModuleList(mods)
         self._plans = {}
 

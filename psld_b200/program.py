@@ -113,7 +113,7 @@ class Plan:
         if self.x3 and (H * W) % 32:        # split-bf16 output goes through the staged epilogue only
             return False
         return (Cb % 64 == 0 and E1 % 64 == 0 and E2 % 64 == 0 and cout % 32 == 0 and pow2(W)
-                and pow2(H) and 4 <= W <= 128 and tuple(e1.shape[:3]) == (N, H, W))
+                and pow2(H) and 4 <= W <= 256 and tuple(e1.shape[:3]) == (N, H, W))
 
     def _release(self, t):
         self.pool.setdefault(tuple(t.shape), []).append(t)
@@ -250,12 +250,16 @@ class Plan:
         self._push(op)
         return y
 
-    def op_fir(self, x, taps, up, down, pad0, pad1, cact=0):
+    def op_fir(self, x, taps, up, down, pad0, pad1, cact=0, f32=False):
+        """upfirdn2d over NHWC ``x``; ``f32``: over a float32 tensor whatever the plan's format."""
         N, H, W, Cc = x.shape
         KH = taps.shape[0]
         OH = (H * up + pad0 + pad1 - KH) // down + 1
         OW = (W * up + pad0 + pad1 - KH) // down + 1
-        if cact and cact < Cc:
+        if f32:
+            cact = 0
+            y = self._new(N, OH, OW, Cc, dtype=torch.float32)
+        elif cact and cact < Cc:
             # only the first `cact` channels carry data (zero-padded network input): the output's
             # padding channels keep the zeros of a dedicated, never-pooled buffer
             y = torch.zeros(N, OH, OW, Cc, dtype=self.adt, device=self.dev)
@@ -267,7 +271,7 @@ class Plan:
         i = op.i
         i[L.FIR_N], i[L.FIR_H], i[L.FIR_W], i[L.FIR_C] = N, H, W, Cc
         i[L.FIR_UP], i[L.FIR_DOWN], i[L.FIR_PAD0], i[L.FIR_PAD1] = up, down, pad0, pad1
-        i[L.FIR_KH], i[L.FIR_DTYPE], i[L.FIR_CACT] = KH, self.acode, cact
+        i[L.FIR_KH], i[L.FIR_DTYPE], i[L.FIR_CACT] = KH, L.F32 if f32 else self.acode, cact
         for j, v in enumerate(taps.reshape(-1)):
             op.f[j] = float(v)
         op.inp[0], op.out[0] = x.data_ptr(), y.data_ptr()
@@ -277,7 +281,8 @@ class Plan:
     def op_conv(self, x1, x2, w_oihw, bias, *, ks, stride=1, pad=None, residual=None,
                 temb_off=-1, scale=1.0, out=None, in_nchw=False, out_nchw_f32=False,
                 hw=None, allow_tc=True, want_stats=True, affine=None, gn_silu=True, ext=None):
-        """y = scale * (conv(cat(x1,x2), w) + bias + temb + residual); w is [Cout, Cin, ks, ks]."""
+        """y = scale * (conv(cat(x1,x2), w) + bias + temb + residual); w is [Cout, Cin, ks, ks].
+        With ``out_nchw_f32`` the residual, if any, is an fp32 NCHW [N, Cout, OH, OW] tensor."""
         pad = ks // 2 if pad is None else pad
         if in_nchw:
             N, C1, H, W = x1.shape
@@ -305,7 +310,7 @@ class Plan:
         i[L.CONV_OUT_LAYOUT] = L.NCHW if out_nchw_f32 else L.NHWC
         i[L.CONV_IN_DTYPE] = L.F32 if in_nchw else self.acode
         i[L.CONV_OUT_DTYPE] = L.F32 if out_nchw_f32 else self.acode
-        i[L.CONV_RES_DTYPE] = self.acode
+        i[L.CONV_RES_DTYPE] = L.F32 if (out_nchw_f32 and residual is not None) else self.acode
         if temb_off >= 0:
             i[L.CONV_TEMB_OFF] = temb_off
             i[L.CONV_TEMB_BSTRIDE] = 0 if self.nt == 1 else self.total_c
@@ -383,9 +388,14 @@ class Plan:
         ks = i[L.CONV_KS]
         same = i[L.CONV_STRIDE] == 1 and ks in (1, 3) and i[L.CONV_PAD] == ks // 2
         down2 = i[L.CONV_STRIDE] == 2 and i[L.CONV_PAD] == 0 and ks == 3 and i[L.CONV_C2] == 0
+        # output rows up to 128 pixels wide are tiled by whole rows; 256-wide rows (stride 1 only) as two
+        # 128-pixel halves
+        ow_max = 256 if same else 128
         ok = (i[L.CONV_IN_DTYPE] in (L.BF16, L.BF16S) and i[L.CONV_IN_LAYOUT] == L.NHWC and (same or down2)
               and i[L.CONV_C1] % 64 == 0 and i[L.CONV_C2] % 64 == 0 and i[L.CONV_COUT] % 32 == 0
-              and pow2(i[L.CONV_OW]) and pow2(i[L.CONV_OH]) and 4 <= i[L.CONV_OW] <= 128)
+              and pow2(i[L.CONV_OW]) and pow2(i[L.CONV_OH]) and 4 <= i[L.CONV_OW] <= ow_max)
+        if i[L.CONV_OUT_LAYOUT] == L.NCHW and op.inp[2]:      # head residual: the fp32 NCHW pyramid
+            ok = ok and i[L.CONV_RES_DTYPE] == L.F32
         if i[L.CONV_IN_DTYPE] == L.BF16S and i[L.CONV_OUT_LAYOUT] == L.NHWC:
             ok = ok and (i[L.CONV_OH] * i[L.CONV_OW]) % 32 == 0
         return L.OK if ok else L.EUNSUPPORTED
@@ -437,6 +447,18 @@ class Plan:
         return o
 
     # ---------------------------------------------------------------- blocks
+    def _resample(self, up):
+        """(taps, up, down, pad0, pad1) of the network's x2 up- or downsampler as an upfirdn2d."""
+        if self.net.fir:
+            if up:      # upsample_2d: upfirdn2d(up=2, pad=(2,1)), taps * factor^2 (:195-224)
+                return _fir_taps(self.net.fir_kernel, 4.0), 2, 1, 2, 1
+            # downsample_2d: upfirdn2d(down=2, pad=(1,1)) (:227-257)
+            return _fir_taps(self.net.fir_kernel, 1.0), 1, 2, 1, 1
+        if up:          # naive_upsample_2d: nearest x2
+            return np.ones((2, 2), np.float32), 2, 1, 1, 0
+        # naive_downsample_2d: 2x2 mean
+        return np.full((2, 2), 0.25, np.float32), 1, 2, 0, 0
+
     def resblock(self, m, x1, x2, temb_off):
         """ResnetBlockBigGANpp.forward (reference layerspp.py:242-274)."""
         net = self.net
@@ -456,20 +478,11 @@ class Plan:
         fir_tmp = []
         if m.up or m.down:
             assert x2 is None
-            if net.fir:
-                if m.up:      # upsample_2d: upfirdn2d(up=2, pad=(2,1)), taps * factor^2 (:195-224)
-                    taps, up, down, p0, p1 = _fir_taps(net.fir_kernel, 4.0), 2, 1, 2, 1
-                else:         # downsample_2d: upfirdn2d(down=2, pad=(1,1)) (:227-257)
-                    taps, up, down, p0, p1 = _fir_taps(net.fir_kernel, 1.0), 1, 2, 1, 1
-            else:
-                if m.up:      # naive_upsample_2d: nearest x2
-                    taps, up, down, p0, p1 = np.ones((2, 2), np.float32), 2, 1, 1, 0
-                else:         # naive_downsample_2d: 2x2 mean
-                    taps, up, down, p0, p1 = np.full((2, 2), 0.25, np.float32), 1, 2, 0, 0
-            a2 = self.op_fir(a, taps, up, down, p0, p1)
+            rs = self._resample(m.up)
+            a2 = self.op_fir(a, *rs)
             self._release(a)
             a = a2
-            xs1 = self.op_fir(x1, taps, up, down, p0, p1)
+            xs1 = self.op_fir(x1, *rs)
             fir_tmp.append(xs1)
         h = self.op_conv(a, None, m.Conv_0.weight, None, ks=3, temb_off=temb_off)  # bias: see temb
         self._release(a)
@@ -605,7 +618,15 @@ class Plan:
             if lvl != net.num_resolutions - 1:
                 m = mods[i]; i += 1
                 h = self.resblock(m, hs[-1], None, offs[id(m)])
-                if net.progressive_input == "residual":
+                if net.progressive_input == "input_skip":
+                    # Combine(sum): the pyramid keeps the input's channels, downsampled once per level;
+                    # h + Conv_0(pyr) is the 1x1 conv with h as its epilogue residual
+                    cact = 8 if (cpad > net.in_ch and net.in_ch <= 8) else 0
+                    pyr = self.op_fir(pyr, *self._resample(False), cact=cact)
+                    cm = mods[i]; i += 1
+                    h = self.op_conv(pyr, None, cm.Conv_0.weight, cm.Conv_0.bias, ks=1, residual=h,
+                                     out=self._new(*h.shape))
+                elif net.progressive_input == "residual":
                     pm = mods[i]; i += 1
                     # conv_downsample_2d: upfirdn2d(pad=(2,2)) then conv(stride 2, pad 0) + bias,
                     # merged with h: (pyr + h)/sqrt(2)   (ncsnpp.py:350-357)
@@ -625,26 +646,47 @@ class Plan:
         h = self.attnblock(mods[i], h); i += 1
         m = mods[i]; i += 1
         h = self.resblock(m, h, None, offs[id(m)])
+        out_pyr = None
         for lvl in reversed(range(net.num_resolutions)):
             for _ in range(net.num_res_blocks + 1):
                 m = mods[i]; i += 1
                 h = self.resblock(m, h, hs.pop(), offs[id(m)])     # cat([h, skip]) is virtual
             if h.shape[2] in net.attn_resolutions:
                 h = self.attnblock(mods[i], h); i += 1
+            if net.progressive == "output_skip":
+                out_pyr = self.head(h, mods[i], mods[i + 1], out_pyr); i += 2
             if lvl != 0:
                 m = mods[i]; i += 1
                 h = self.resblock(m, h, None, offs[id(m)])
         assert not hs
-        if self._gn_fusable(h, None, 64):
-            # final act(GroupNorm(h)) -> conv3x3 -> fp32 NCHW eps as one GroupNorm-on-load conv
-            aff = self.op_gn(h, None, mods[i], True, h.shape[1] * h.shape[2], affine_only=True); i += 1
-            self.eps = self.op_conv(h, None, mods[i].weight, mods[i].bias, ks=3, out_nchw_f32=True,
-                                    affine=aff); i += 1
+        if net.progressive == "output_skip":
+            self.eps = out_pyr
         else:
-            a = self.op_gn(h, None, mods[i], True, h.shape[1] * h.shape[2]); i += 1
-            self.eps = self.op_conv(a, None, mods[i].weight, mods[i].bias, ks=3, out_nchw_f32=True); i += 1
+            self.eps = self.head(h, mods[i], mods[i + 1], None); i += 2
         assert i == len(mods), (i, len(mods))
         self._finish_stat_arenas(zero_ops)
+
+    def head(self, h, gn, conv, pyr):
+        """conv3x3(act(GroupNorm(h))) -> fp32 NCHW [B, out_ch, H, W], plus the x2-upsampled output
+        pyramid ``pyr`` of the level below when given (progressive=output_skip, ncsnpp.py:405-418).
+        The pyramid is upsampled as B*out_ch single-channel planes and added in the conv epilogue."""
+        HW = h.shape[1] * h.shape[2]
+        res = None
+        if pyr is not None:
+            B, Cc, H, W = pyr.shape
+            res = self.op_fir(pyr.view(B * Cc, H, W, 1), *self._resample(True), f32=True)
+            res = res.view(B, Cc, 2 * H, 2 * W)
+        if self._gn_fusable(h, None, 64):
+            # act(GroupNorm(h)) -> conv3x3 -> fp32 NCHW as one GroupNorm-on-load conv
+            aff = self.op_gn(h, None, gn, True, HW, affine_only=True)
+            out = self.op_conv(h, None, conv.weight, conv.bias, ks=3, out_nchw_f32=True, affine=aff,
+                               residual=res)
+            self._release_affine(aff)
+        else:
+            a = self.op_gn(h, None, gn, True, HW)
+            out = self.op_conv(a, None, conv.weight, conv.bias, ks=3, out_nchw_f32=True, residual=res)
+            self._release(a)
+        return out
 
     # ---------------------------------------------------------------- execution
     def run(self, stream=None):
