@@ -340,7 +340,15 @@ enum { PSLD_CONV_N = 0, PSLD_CONV_H, PSLD_CONV_W, PSLD_CONV_C1, PSLD_CONV_C2, PS
  *   PROJ = 1 (PSLD_ENGINE_TC, HW % 128 == 0): the block's output projection and skip connection are
  *   fused (layerspp.py:87-91): out[0] = (NIN_3(o) + x) * f[1] with in[1] = NIN_3 weight bf16
  *   [C out, C in], in[2] = bias f32 [C] or NULL, in[3] = x [N, HW, C]; out[1] = optional GroupNorm
- *   statistics accumulator of out[0] (as for PSLD_OP_CONV)                                 */
+ *   statistics accumulator of out[0] (as for PSLD_OP_CONV)
+ *   Accepted shapes per engine:
+ *     PSLD_ENGINE_TC (DTYPE bf16 or split bf16): C in {64, 128, 192, 256} and HW in {64, 128, 256}
+ *       (all keys of a query tile in one TMEM accumulator) or HW % 128 == 0 with HW >= 512 (keys
+ *       streamed in tiles with an online softmax).  Other shapes: psld_op_prepare returns
+ *       PSLD_EUNSUPPORTED.
+ *     PSLD_ENGINE_SIMT (any DTYPE, PROJ = 0): any HW and C.  Keys are processed in one chunk when
+ *       32 x (HW + 1) fp32 scores fit in shared memory (HW <= 1518), otherwise in chunks with an
+ *       online softmax.                                                                        */
 enum { PSLD_ATTN_N = 0, PSLD_ATTN_HW, PSLD_ATTN_C, PSLD_ATTN_DTYPE, PSLD_ATTN_PROJ };
 
 /* Standalone PSLD_OP_AXPBY: out = a * x + b * y over n floats (y may be NULL). */

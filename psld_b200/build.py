@@ -8,7 +8,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.environ.get("PSLD_B200_LIB") or os.path.join(HERE, "libpsld_b200.so")
-SOURCES = ["capi.cu", "phase_space.cu", "net_simt.cu", "conv_simt.cu", "conv_tc.cu", "conv_gn_tc.cu", "attn_tc.cu"]
+SOURCES = ["capi.cu", "phase_space.cu", "net_simt.cu", "conv_simt.cu", "conv_tc.cu", "conv_gn_tc.cu", "attn_tc.cu",
+           "attn_stream_tc.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",

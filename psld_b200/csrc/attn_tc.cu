@@ -445,14 +445,6 @@ extern "C" __attribute__((visibility("default"))) int psld_debug_attn_trace(long
 #endif
 
 // ---------------------------------------------------------------- host side
-static int encode_qkv_map(CUtensorMap* tm, const void* ptr, int N, int HW, int C3, int rows) {
-  const cuuint64_t dims[3] = {(cuuint64_t)C3, (cuuint64_t)HW, (cuuint64_t)N};
-  const cuuint64_t strides[2] = {(cuuint64_t)C3 * 2, (cuuint64_t)HW * C3 * 2};
-  const cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  return encode_bf16_map(tm, ptr, 3, dims, strides, box, estr, "qkv");
-}
-
 int prepare_attn_tc(psld_op& op) {
   const int N = op.i[PSLD_ATTN_N], HW = op.i[PSLD_ATTN_HW], C = op.i[PSLD_ATTN_C];
   auto unsupported = [&](const char* why) {
@@ -464,7 +456,8 @@ int prepare_attn_tc(psld_op& op) {
   const bool x3 = adt == PSLD_BF16S;
   const int cm = x3 ? 2 : 1;
   if (C % 64 || C < 64 || C > 256) return unsupported("C must be 64..256, multiple of 64");
-  if (HW != 64 && HW != 128 && HW != 256) return unsupported("HW must be 64, 128 or 256");
+  if (attn_streams_keys(HW)) return prepare_attn_stream_tc(op);
+  if (HW != 64 && HW != 128 && HW != 256) return unsupported("HW must be 64, 128, 256 or a multiple of 128 from 512");
   if (!op.in[0] || !op.out[0]) { set_error("attn_tc: null pointer"); return PSLD_EINVAL; }
   AttnTcState* st = new (std::nothrow) AttnTcState();
   if (!st) { set_error("attn_tc: out of host memory"); return PSLD_ECUDA; }
@@ -531,6 +524,7 @@ int prepare_attn_tc(psld_op& op) {
 }
 
 int release_attn_tc(psld_op& op) {
+  if (attn_streams_keys(op.i[PSLD_ATTN_HW])) return release_attn_stream_tc(op);
   if (op.aux) {
     delete (AttnTcState*)op.aux;
     op.aux = nullptr;
@@ -539,6 +533,7 @@ int release_attn_tc(psld_op& op) {
 }
 
 int run_attn_tc(const psld_op& op, cudaStream_t s) {
+  if (attn_streams_keys(op.i[PSLD_ATTN_HW])) return run_attn_stream_tc(op, s);
   const AttnTcState* st = (const AttnTcState*)op.aux;
   PSLD_CHECK_ARG(st != nullptr, "attn_tc: op not prepared (call psld_op_prepare)");
 #define ATTN_LAUNCH(PROJ, X3)                                                                  \

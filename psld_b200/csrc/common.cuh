@@ -214,6 +214,12 @@ int run_conv_gn_tc(const psld_op& op, cudaStream_t s);
 int prepare_attn_tc(psld_op& op);
 int release_attn_tc(psld_op& op);
 int run_attn_tc(const psld_op& op, cudaStream_t s);
+// tensor-core attention over more than 256 tokens runs the key-streaming kernel (attn_stream_tc.cu);
+// prepare_attn_tc hands it the shapes it takes (HW % 128 == 0, HW >= 512)
+inline bool attn_streams_keys(int HW) { return HW > 256; }
+int prepare_attn_stream_tc(psld_op& op);
+int release_attn_stream_tc(psld_op& op);
+int run_attn_stream_tc(const psld_op& op, cudaStream_t s);
 
 int launch_step_inc(int* step_ptr, cudaStream_t s);
 int launch_sscs_table(void* u, int state_dtype, float* net_in, const float* eps,

@@ -202,111 +202,140 @@ int run_conv_simt(const psld_op& op, cudaStream_t s) {
 }
 
 // ======================================================================== attention (SIMT)
-// One CTA = one sample x 32 queries.  S = scale * Q K^T (all HW keys) lives in shared memory,
-// softmax over keys, O = P V.  q|k|v are packed along the channel axis of one [N,HW,3C] tensor
-// produced by a single fused NIN GEMM.
+// One CTA = one sample x 32 queries.  q|k|v are packed along the channel axis of one [N,HW,3C] tensor
+// produced by a single fused NIN GEMM.  Keys are taken in chunks of KC: S = scale * Q K^T of a chunk
+// lives in shared memory ([TQ][KC + 1] floats).
+//   KC >= HW (every score row fits, HW <= 1518): one pass with an exact softmax, P = softmax(S),
+//            O = P V (the S block is computed once and reused by every 256-channel block)
+//   KC <  HW: online softmax per chunk: m_new = max(m, rowmax), P = exp(S - m_new),
+//            l = l * exp(m - m_new) + rowsum(P), O = O * exp(m - m_new) + P V;  out = O / l.
+//            Each 256-channel block recomputes its chunks' S (O stays in registers).
 constexpr int TQ = 32;
+constexpr int ATTN_TILE = TQ * 33 + 256 * 33 > 32 * 256 ? TQ * 33 + 256 * 33 : 32 * 256;   // floats
 
 template <typename T>
 __global__ void __launch_bounds__(256)
-attn_simt_kernel(const T* __restrict__ qkv, T* __restrict__ out, int HW, int C, float scale) {
+attn_simt_kernel(const T* __restrict__ qkv, T* __restrict__ out, int HW, int C, int KC, float scale) {
   pdl_wait();
   extern __shared__ float smem[];
-  float* S = smem;                               // [TQ][HW + 1]
-  float* buf = smem + TQ * (HW + 1);             // tile buffers
+  const int ldS = KC + 1;
+  float* S = smem;                               // [TQ][KC + 1]
+  float* buf = smem + TQ * ldS;                  // tile buffers
+  float* rowst = buf + ATTN_TILE;                // KC < HW: [running max | running sum | rescale][TQ]
+  const bool one = KC >= HW;
   const int n = blockIdx.y, q0 = blockIdx.x * TQ;
   const int tid = threadIdx.x;
   const int tq = tid >> 3, tk = tid & 7;
   const int lo = 3 * C;                          // split-bf16 lo offset of a q|k|v row
   const int ld = lo * Elt<T>::kMul;
   const T* base = qkv + (int64_t)n * HW * ld;
+  float* Qs = buf;                 // phase 1: [TQ][33]
+  float* Ks = buf + TQ * 33;       //          [256][33]
+  float* Vs = buf;                 // phase 3: [32][256]
 
-  // ---- phase 1: S = scale * Q K^T, key blocks of 256, channel chunks of 32
-  float* Qs = buf;                 // [TQ][33]
-  float* Ks = buf + TQ * 33;       // [256][33]
-  for (int kb = 0; kb < HW; kb += 256) {
-    float acc[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-    for (int c0 = 0; c0 < C; c0 += 32) {
-      for (int e = tid; e < TQ * 32; e += 256) {
-        const int r = e >> 5, cc = e & 31;
-        const int q = q0 + r;
-        Qs[r * 33 + cc] = (q < HW && c0 + cc < C) ? ld_elt<T>(base + (int64_t)q * ld + c0 + cc, lo) : 0.f;
-      }
-      for (int e = tid; e < 256 * 32; e += 256) {
-        const int r = e >> 5, cc = e & 31;
-        const int key = kb + r;
-        Ks[r * 33 + cc] =
-            (key < HW && c0 + cc < C) ? ld_elt<T>(base + (int64_t)key * ld + C + c0 + cc, lo) : 0.f;
-      }
-      __syncthreads();
-#pragma unroll 4
-      for (int cc = 0; cc < 32; ++cc) {
-        const float qv = Qs[tq * 33 + cc];
-#pragma unroll
-        for (int i = 0; i < 32; ++i) acc[i] = fmaf(qv, Ks[(tk + 8 * i) * 33 + cc], acc[i]);
-      }
-      __syncthreads();
-    }
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-      const int key = kb + tk + 8 * i;
-      if (key < HW) S[tq * (HW + 1) + key] = acc[i] * scale;   // einsum then * C^-0.5 (layerspp.py:82)
-    }
-  }
-  __syncthreads();
-
-  // ---- phase 2: row softmax (F.softmax over keys, layerspp.py:84)
-  {
-    const int warp = tid >> 5, lane = tid & 31;
-    for (int r = warp; r < TQ; r += 8) {
-      float* row = S + r * (HW + 1);
-      float mx = -INFINITY;
-      for (int k = lane; k < HW; k += 32) mx = fmaxf(mx, row[k]);
-#pragma unroll
-      for (int d = 16; d > 0; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-      float sum = 0.f;
-      for (int k = lane; k < HW; k += 32) {
-        const float e = expf(row[k] - mx);
-        row[k] = e;
-        sum += e;
-      }
-#pragma unroll
-      for (int d = 16; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
-      const float inv = 1.0f / sum;
-      for (int k = lane; k < HW; k += 32) row[k] *= inv;
-    }
-  }
-  __syncthreads();
-
-  // ---- phase 3: O = P V, channel blocks of 256, key chunks of 32
-  float* Vs = buf;                 // [32][256]
   for (int cb = 0; cb < C; cb += 256) {
     float acc[32];
 #pragma unroll
     for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-    for (int k0 = 0; k0 < HW; k0 += 32) {
-      for (int e = tid; e < 32 * 256; e += 256) {
-        const int r = e >> 8, cc = e & 255;
-        const int key = k0 + r;
-        Vs[e] = (key < HW && cb + cc < C) ? ld_elt<T>(base + (int64_t)key * ld + 2 * C + cb + cc, lo) : 0.f;
-      }
-      __syncthreads();
-#pragma unroll 4
-      for (int kk = 0; kk < 32; ++kk) {
-        const float pv = (k0 + kk < HW) ? S[tq * (HW + 1) + k0 + kk] : 0.f;
+    for (int kc0 = 0; kc0 < HW; kc0 += KC) {
+      const int kn = HW - kc0 < KC ? HW - kc0 : KC;
+      if (!one || cb == 0) {
+        // ---- phase 1: S = scale * Q K^T over the chunk's keys, key blocks of 256, channel chunks of 32
+        for (int kb = 0; kb < kn; kb += 256) {
+          float sacc[32];
 #pragma unroll
-        for (int i = 0; i < 32; ++i) acc[i] = fmaf(pv, Vs[kk * 256 + tk + 8 * i], acc[i]);
+          for (int i = 0; i < 32; ++i) sacc[i] = 0.f;
+          for (int c0 = 0; c0 < C; c0 += 32) {
+            for (int e = tid; e < TQ * 32; e += 256) {
+              const int r = e >> 5, cc = e & 31;
+              const int q = q0 + r;
+              Qs[r * 33 + cc] = (q < HW && c0 + cc < C) ? ld_elt<T>(base + (int64_t)q * ld + c0 + cc, lo) : 0.f;
+            }
+            for (int e = tid; e < 256 * 32; e += 256) {
+              const int r = e >> 5, cc = e & 31;
+              const int key = kb + r;
+              Ks[r * 33 + cc] = (key < kn && c0 + cc < C)
+                                    ? ld_elt<T>(base + (int64_t)(kc0 + key) * ld + C + c0 + cc, lo) : 0.f;
+            }
+            __syncthreads();
+#pragma unroll 4
+            for (int cc = 0; cc < 32; ++cc) {
+              const float qv = Qs[tq * 33 + cc];
+#pragma unroll
+              for (int i = 0; i < 32; ++i) sacc[i] = fmaf(qv, Ks[(tk + 8 * i) * 33 + cc], sacc[i]);
+            }
+            __syncthreads();
+          }
+#pragma unroll
+          for (int i = 0; i < 32; ++i) {
+            const int key = kb + tk + 8 * i;
+            if (key < kn) S[tq * ldS + key] = sacc[i] * scale;   // einsum then * C^-0.5 (layerspp.py:82)
+          }
+        }
+        __syncthreads();
+
+        // ---- phase 2: row softmax (F.softmax over keys, layerspp.py:84)
+        {
+          const int warp = tid >> 5, lane = tid & 31;
+          for (int r = warp; r < TQ; r += 8) {
+            float* row = S + r * ldS;
+            float mx = -INFINITY;
+            for (int k = lane; k < kn; k += 32) mx = fmaxf(mx, row[k]);
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, d));
+            const float m_old = (one || kc0 == 0) ? -INFINITY : rowst[r];
+            const float m_new = fmaxf(m_old, mx);
+            float sum = 0.f;
+            for (int k = lane; k < kn; k += 32) {
+              const float e = expf(row[k] - m_new);
+              row[k] = e;
+              sum += e;
+            }
+#pragma unroll
+            for (int d = 16; d > 0; d >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, d);
+            if (one) {
+              const float inv = 1.0f / sum;
+              for (int k = lane; k < kn; k += 32) row[k] *= inv;
+            } else if (lane == 0) {
+              const float a = kc0 == 0 ? 0.f : expf(m_old - m_new);
+              rowst[r] = m_new;
+              rowst[TQ + r] = (kc0 == 0 ? 0.f : rowst[TQ + r] * a) + sum;
+              rowst[2 * TQ + r] = a;
+            }
+          }
+        }
+        __syncthreads();
       }
-      __syncthreads();
+
+      // ---- phase 3: O (+)= P V over the chunk's keys, key chunks of 32
+      if (!one) {
+        const float a = rowst[2 * TQ + tq];
+#pragma unroll
+        for (int i = 0; i < 32; ++i) acc[i] *= a;
+      }
+      for (int k0 = 0; k0 < kn; k0 += 32) {
+        for (int e = tid; e < 32 * 256; e += 256) {
+          const int r = e >> 8, cc = e & 255;
+          const int key = k0 + r;
+          Vs[e] = (key < kn && cb + cc < C) ? ld_elt<T>(base + (int64_t)(kc0 + key) * ld + 2 * C + cb + cc, lo) : 0.f;
+        }
+        __syncthreads();
+#pragma unroll 4
+        for (int kk = 0; kk < 32; ++kk) {
+          const float pv = (k0 + kk < kn) ? S[tq * ldS + k0 + kk] : 0.f;
+#pragma unroll
+          for (int i = 0; i < 32; ++i) acc[i] = fmaf(pv, Vs[kk * 256 + tk + 8 * i], acc[i]);
+        }
+        __syncthreads();
+      }
     }
     const int q = q0 + tq;
     if (q < HW) {
+      const float inv = one ? 1.0f : 1.0f / rowst[TQ + tq];
 #pragma unroll
       for (int i = 0; i < 32; ++i) {
         const int c = cb + tk + 8 * i;
-        if (c < C) st_elt<T>(out + ((int64_t)n * HW + q) * (C * Elt<T>::kMul) + c, acc[i], C);
+        if (c < C) st_elt<T>(out + ((int64_t)n * HW + q) * (C * Elt<T>::kMul) + c, one ? acc[i] : acc[i] * inv, C);
       }
     }
   }
@@ -316,26 +345,31 @@ int run_attn_simt(const psld_op& op, cudaStream_t s) {
   const int N = op.i[PSLD_ATTN_N], HW = op.i[PSLD_ATTN_HW], C = op.i[PSLD_ATTN_C];
   const int dt = op.i[PSLD_ATTN_DTYPE];
   PSLD_CHECK_ARG(N > 0 && HW > 0 && C > 0 && op.in[0] && op.out[0], "attn: bad arguments");
-  const size_t tile = (size_t)TQ * 33 + 256 * 33 > (size_t)32 * 256 ? (size_t)TQ * 33 + 256 * 33
-                                                                     : (size_t)32 * 256;
-  const size_t smem = ((size_t)TQ * (HW + 1) + tile) * sizeof(float);
-  PSLD_CHECK_ARG(smem <= 227 * 1024, "attn: HW=%d needs %zu B shared memory", HW, smem);
+  // the whole score row in one chunk when it fits; otherwise the largest multiple of 256 keys that fits
+  // beside the row statistics
+  constexpr size_t kMaxSmem = 227 * 1024;
+  int KC = HW;
+  size_t smem = ((size_t)TQ * (HW + 1) + ATTN_TILE) * sizeof(float);
+  if (smem > kMaxSmem) {
+    KC = (int)((kMaxSmem / sizeof(float) - ATTN_TILE - 3 * TQ) / TQ - 1) / 256 * 256;
+    smem = ((size_t)TQ * (KC + 1) + ATTN_TILE + 3 * TQ) * sizeof(float);
+  }
   dim3 grid((unsigned)ceil_div(HW, TQ), (unsigned)N);
   if (dt == PSLD_BF16) {
     PSLD_CHECK_CUDA(cudaFuncSetAttribute(attn_simt_kernel<__nv_bfloat16>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     launch_pdl(attn_simt_kernel<__nv_bfloat16>, dim3(grid), dim3(256), smem, s, 1, (const __nv_bfloat16*)op.in[0],
-                                                           (__nv_bfloat16*)op.out[0], HW, C, op.f[0]);
+               (__nv_bfloat16*)op.out[0], HW, C, KC, op.f[0]);
   } else if (dt == PSLD_BF16S) {
     PSLD_CHECK_CUDA(cudaFuncSetAttribute(attn_simt_kernel<bf16s>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     launch_pdl(attn_simt_kernel<bf16s>, dim3(grid), dim3(256), smem, s, 1, (const bf16s*)op.in[0],
-               (bf16s*)op.out[0], HW, C, op.f[0]);
+               (bf16s*)op.out[0], HW, C, KC, op.f[0]);
   } else {
     PSLD_CHECK_CUDA(cudaFuncSetAttribute(attn_simt_kernel<float>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    launch_pdl(attn_simt_kernel<float>, dim3(grid), dim3(256), smem, s, 1, (const float*)op.in[0], (float*)op.out[0], HW, C,
-                                                   op.f[0]);
+    launch_pdl(attn_simt_kernel<float>, dim3(grid), dim3(256), smem, s, 1, (const float*)op.in[0], (float*)op.out[0],
+               HW, C, KC, op.f[0]);
   }
   PSLD_CHECK_LAUNCH();
   return PSLD_OK;

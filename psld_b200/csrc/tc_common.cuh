@@ -165,4 +165,14 @@ static inline int encode_bf16_map(CUtensorMap* tm, const void* ptr, int rank, co
   return PSLD_OK;
 }
 
+// q|k|v of the attention block: one [N, HW, C3] bf16 tensor (C3 = 3C, split bf16: 6C), boxes of
+// 64 channels x `rows` tokens of one sample.
+static inline int encode_qkv_map(CUtensorMap* tm, const void* ptr, int N, int HW, int C3, int rows) {
+  const cuuint64_t dims[3] = {(cuuint64_t)C3, (cuuint64_t)HW, (cuuint64_t)N};
+  const cuuint64_t strides[2] = {(cuuint64_t)C3 * 2, (cuuint64_t)HW * C3 * 2};
+  const cuuint32_t box[3] = {64, (cuuint32_t)rows, 1};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  return encode_bf16_map(tm, ptr, 3, dims, strides, box, estr, "qkv");
+}
+
 }  // namespace psld

@@ -16,7 +16,12 @@ Supported configuration space (the BASELINE configs, the shipped sampling script
 high-resolution NCSN++ configurations of the score-SDE family): ``resblock_type=biggan``,
 ``progressive in {none,output_skip}``, ``progressive_input in {none,residual,input_skip}``,
 ``progressive_combine=sum``, ``embedding_type in {fourier,positional}``, ``fir in {True,False}``
-(``progressive_input=residual`` needs ``fir=True``), ``nonlinearity=swish``.
+(``progressive_input=residual`` needs ``fir=True``), ``nonlinearity=swish``, and any
+``attn_resolutions``.  Attention runs on the tensor cores (``bf16``, ``bf16x3``) at C = 64..256
+(multiple of 64) over 64, 128 or 256 tokens (all keys in one accumulator) or any multiple of 128
+tokens from 512 (32x32 maps and larger: keys streamed with an online softmax); other shapes and
+the ``fp32`` tier run it on the CUDA cores, which stream keys in chunks when a score row does not
+fit in shared memory, so every map size runs.
 """
 from __future__ import annotations
 

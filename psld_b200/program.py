@@ -400,6 +400,12 @@ class Plan:
             ok = ok and (i[L.CONV_OH] * i[L.CONV_OW]) % 32 == 0
         return L.OK if ok else L.EUNSUPPORTED
 
+    @staticmethod
+    def _attn_tc_eligible(HW, Cc):
+        """Mirrors prepare_attn_tc: attn_tc holds all keys of a query tile (64, 128, 256 tokens),
+        attn_stream_tc streams them (multiples of 128 from 512); C > 256 would not fit TMEM."""
+        return Cc % 64 == 0 and 64 <= Cc <= 256 and (HW in (64, 128, 256) or (HW % 128 == 0 and HW >= 512))
+
     def op_attn(self, qkv, HW, Cc, proj=None):
         """proj = (W3 [out, in], bias, x, scale, out): the output projection + skip connection are
         fused into the tensor-core attention kernel; returns None if that is not possible."""
@@ -407,7 +413,8 @@ class Plan:
         op.i[L.ATTN_N], op.i[L.ATTN_HW], op.i[L.ATTN_C], op.i[L.ATTN_DTYPE] = self.B, HW, Cc, self.acode
         op.f[0] = float(int(Cc) ** (-0.5))
         op.inp[0] = qkv.data_ptr()
-        fusable = Cc % 64 == 0 and 64 <= Cc <= 256 and HW in (128, 256)
+        tc_ok = self._attn_tc_eligible(HW, Cc)
+        fusable = tc_ok and HW % 128 == 0
         if proj is not None:
             if not (self.tc and fusable):
                 return None
@@ -427,7 +434,7 @@ class Plan:
         if self.tc:
             op.engine = L.ENGINE_TC
             if self.dry:
-                rc = L.OK if (Cc % 64 == 0 and 64 <= Cc <= 256 and HW in (64, 128, 256)) else L.EUNSUPPORTED
+                rc = L.OK if tc_ok else L.EUNSUPPORTED
             else:
                 rc = self.lib.psld_op_prepare(C.byref(op))
             if rc == L.EUNSUPPORTED:
