@@ -98,6 +98,20 @@ typedef struct {
   double gs_x, gs_m;             /* g_x sqrt(dt), g_m sqrt(dt)  (0 for denoise)         */
 } psld_score_step;
 
+/* In-kernel noise (every entry point below that takes `seed` and `step`).  One draw is
+ * Philox4x32-10 with key (seed lo, seed hi) and counter (index lo, index hi, stream lo, stream hi),
+ * turned into 4 normals by Box-Muller: u0 = min((f32(r.x) + 0.5) 2^-32, 1 - 2^-24), u1 = f32(r.y) 2^-32
+ * (u2, u3 likewise from r.z, r.w), angle 2 pi (u1 - 0.5) in [-pi, pi), normals
+ * (ra cos a, ra sin a, rb cos b, rb sin b) with ra = sqrt(-2 log u0).  (stream, index) per entry point:
+ *   PSLD state [B,2C,H,W] (psld_sscs_update, psld_em_update[_guided], psld_prior_sample): the 4 pairs
+ *     j..j+3 (j % 4 == 0) of sample b form vector v = b chw/4 + j/4; x[j..j+3] take draw index 2v,
+ *     m[j..j+3] index 2v + 1.  Streams: SSCS stage slots 2 step (HALF_A), 2 step + 1 (HALF_B),
+ *     2 step + 2 (HALF_C, = HALF_A of step + 1); Euler-Maruyama: step; prior: 2^64 - 1.
+ *   psld_vp_em_update: stream step, index v = element / 4 of the flat [n] state.
+ *   psld_inpaint_combine: streams (step << 2) | 2^62 | {0, 1, 2} for (z_m0, e_x, e_m), index
+ *     v = element / 4 of the flat [B,C,H,W] tensor.
+ * tests/_philox.py restates this on the host; tests/test_gpu_philox_paths.py pins it. */
+
 /* stage bits for psld_sscs_update */
 #define PSLD_STAGE_HALF_A 1 /* u <- A_a u + L_a z_a            (first half of a step) */
 #define PSLD_STAGE_SCORE 2  /* Euler score step with eps                              */
@@ -115,8 +129,9 @@ typedef struct {
  *   net_in       : optional fp32 copy of u_out (the next score_fn input, sde.py:320), or NULL.
  *   eps          : fp32 NCHW network output [B, 2C or C, H, W]; required with STAGE_SCORE.
  *   z_a/z_b/z_c  : pre-drawn fp32 N(0,1) noise [B,2C,H,W] per stage (parity mode).  When a
- *                  needed pointer is NULL the kernel draws from Philox4x32-10 keyed by
- *                  (seed, stream id = stage slot of `step`, pair index)  (throughput mode).
+ *                  needed pointer is NULL the kernel draws from Philox4x32-10 (throughput mode),
+ *                  see "In-kernel noise" below: stream 2 step (HALF_A), 2 step + 1 (HALF_B),
+ *                  2 step + 2 (HALF_C).
  *   B, chw       : batch and C*H*W (pairs per sample); chw % 4 == 0.
  * Algorithmic HBM bytes per pair (fp32 state): 8 (u in) + 8 (u out) + 8 (eps) + 8 per
  * pre-drawn noise tensor [+ 8 net_in]; Philox mode drops the noise reads.
@@ -152,8 +167,9 @@ PSLD_API int psld_em_update_guided(void* u_out, const void* u_in, int state_dtyp
  *   x_k  = mu_x + c11 e_x + c12 e_m ;  m_k = mu_m + c21 e_x + c22 e_m   (mean_only: x_k = mu_x, ...)
  *   x    = x (1 - mask) + x_k mask ;  m = m (1 - mask) + m_k mask        (sde.py:175-178)
  * u: [B,2C,H,W] state (in place, f64 or f32); x0, mask: fp32 [B,C,H,W]; z_m0 [B,C,H,W] and
- * z_eps [B,2C,H,W] are pre-drawn N(0,1) tensors or NULL (both NULL: Philox4x32-10 keyed by
- * (seed, step)); net_in (optional): fp32 copy of the new state for the next score_fn call. */
+ * z_eps [B,2C,H,W] are pre-drawn N(0,1) tensors or NULL (both NULL: in-kernel noise, three streams
+ * per step, see above; z_eps alone: z_m0 = 0); net_in (optional): fp32 copy of the new state for the
+ * next score_fn call. */
 typedef struct psld_inpaint_step {
   double a_xx, a_xm, a_mx, a_mm;
   double c11, c12, c21, c22;

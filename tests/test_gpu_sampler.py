@@ -251,16 +251,18 @@ def test_cuda_graph_replay_equals_host_loop(kind, fuse, merge):
 
 
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
-def test_image_quantisation_bit_exact(dtype):
+@pytest.mark.parametrize("B,H", [(7, 32), (256, 32), (64, 64), (32, 256)])
+def test_image_quantisation_bit_exact(dtype, B, H):
     """Fused writer arithmetic (drop momentum, x*0.5+0.5, *255, clip, truncate) == the reference's
-    numpy sequence, bit for bit (integer output)."""
+    numpy sequence, bit for bit (integer output), at the benchmark's batches and past the grid cap."""
     from psld_b200 import samples_to_uint8
     g = torch.Generator().manual_seed(5)
-    st = (torch.randn(7, 6, 32, 32, generator=g, dtype=torch.float64) * 1.3).to(dtype)
+    st = (torch.randn(B, 6, H, H, generator=g, dtype=torch.float64) * 1.3).to(dtype)
     st[0, 0, 0, :4] = torch.tensor([-1.0, 1.0, 0.0, 0.999999], dtype=dtype)   # edges of the range
+    st[-1, 2, -1, -4:] = torch.tensor([-1.0, 1.0, 0.0, 0.999999], dtype=dtype)
     got = samples_to_uint8(st.cuda()).cpu().numpy()
     ref = O.images_uint8(st)
-    assert got.shape == ref.shape == (7, 32, 32, 3) and got.dtype == ref.dtype
+    assert got.shape == ref.shape == (B, H, H, 3) and got.dtype == ref.dtype
     assert (got == ref).all()
 
 

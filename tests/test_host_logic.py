@@ -282,3 +282,96 @@ def test_guided_program_vs_golden(golden_dir):
         ClassifierFreeGuidance(cond=nets[0], uncond=nets[0], weight=1.0)
     with pytest.raises(RuntimeError, match="CUDA"):
         m(torch.zeros(1, 6, 32, 32), torch.ones(1))
+
+
+# ------------------------------------------------------------------ in-kernel noise: host reference
+@pytest.mark.parametrize("counter,key,want", [
+    ((0, 0, 0, 0), (0, 0), (0x6627e8d5, 0xe169c58d, 0xbc57ac4c, 0x9b00dbd8)),
+    ((0xffffffff,) * 4, (0xffffffff,) * 2, (0x408f276d, 0x41c83b0e, 0xa20bc7c6, 0x6d5451fd)),
+    ((0x243f6a88, 0x85a308d3, 0x13198a2e, 0x03707344), (0xa4093822, 0x299f31d0),
+     (0xd16cfe09, 0x94fdcceb, 0x5001e420, 0x24126ea1)),
+    ((6, 0, 3, 0), (7, 0), (0x548d6e57, 0xd5e0b3d0, 0x332db457, 0x95ca6e68)),   # index 6, stream 3, seed 7
+])
+def test_philox_host_reference_known_answers(counter, key, want):
+    """tests/_philox.py is Philox4x32-10: the Random123 / cuRAND known-answer vectors, and the
+    (seed, stream, index) -> (key, counter) packing of the device's Philox::draw."""
+    import _philox as P
+    assert tuple(int(w) for w in P.philox4x32_10(counter, key)) == want
+    idx = (counter[1] << 32) | counter[0]
+    stream = (counter[3] << 32) | counter[2]
+    seed = (key[1] << 32) | key[0]
+    assert tuple(int(w) for w in P.draw(seed, stream, idx)) == want
+
+
+def test_philox_host_index_rules():
+    """The whole-tensor and single-pair forms of each index rule agree, and the rules keep the x and
+    m halves, the SSCS stages and the inpainting draws on distinct (stream, index) pairs."""
+    import _philox as P
+    from psld_b200.distributed import call_seed
+    seed, B, chw = call_seed(7, 1, 3), 3, 20
+    assert seed >> 32                                      # the high key word is exercised
+    zx, zm = P.pair_normals(seed, P.sscs_stream(70001, "b"), B, chw)
+    b, j = np.meshgrid(np.arange(B), np.arange(chw), indexing="ij")
+    ax, am = P.pair_normals_at(seed, P.sscs_stream(70001, "b"), b, j, chw)
+    assert np.array_equal(zx, ax) and np.array_equal(zm, am)
+    # x of vector v is draw 2v, m is draw 2v + 1
+    assert np.array_equal(zx[1, 8:12], P.normal4(seed, 2 * 70001 + 1, 2 * (chw // 4 + 2)))
+    assert np.array_equal(zm[1, 8:12], P.normal4(seed, 2 * 70001 + 1, 2 * (chw // 4 + 2) + 1))
+    assert P.sscs_stream(5, "a") == 10 and P.sscs_stream(5, "c") == P.sscs_stream(6, "a") == 12
+    assert P.inpaint_stream(3, 2) == (3 << 2) | (1 << 62) | 2
+    f = P.flat_normals(seed, P.inpaint_stream(3, 1), B * chw)
+    assert np.array_equal(f, P.flat_normals_at(seed, P.inpaint_stream(3, 1), np.arange(B * chw)))
+    # standard normal to sampling accuracy, and the tail stays inside the device's 6.77 sigma
+    z = P.flat_normals(seed, 9, 1 << 20)
+    assert abs(z.mean()) < 5e-3 and abs(z.var() - 1) < 5e-3 and np.abs(z).max() < 6.77
+
+
+def _merge_ref(hb, hc):
+    """One draw for two consecutive half-steps, from the oracle's algebra: A = A_c A_b and
+    L L^T = A_c L_b L_b^T A_c^T + L_c L_c^T."""
+    (ab, lb), (ac, lc) = ([np.array(v, dtype=np.float64).reshape(2, 2) for v in h] for h in (hb, hc))
+    S = ac @ lb @ lb.T @ ac.T + lc @ lc.T
+    return ac @ ab, S
+
+
+@pytest.mark.parametrize("n_steps,stride,sde", [(1000, "uniform", {}), (1000, "quadratic", {}),
+                                                (1000, "uniform", dict(nu=4.0, gamma=0.0)),
+                                                (4000, "uniform", dict(nu=4.0, gamma=0.0)),
+                                                (1000, "uniform", dict(beta_min=0.5, beta_max=12.0))])
+def test_merged_half_steps_identity(n_steps, stride, sde):
+    """merge_noise tables (half B of step i and half A of step i+1 as one Gaussian draw) satisfy, row
+    by row, A_bc = A_c A_b and L_bc L_bc^T = A_c L_b L_b^T A_c^T + L_c L_c^T with L_bc lower-triangular,
+    computed from oracle.PSLDScalars.half_step; the last row and the other halves stay unmerged.
+    (With a constant beta on a uniform grid A_b = A_c, so the linear-beta row pins A_c against A_b.)"""
+    from psld_b200 import cifar10_config
+    cfg = cifar10_config(n_discrete_steps=n_steps, stride_type=stride)
+    cfg.model.sde.update(sde)
+    s = O.PSLDScalars(cfg)
+    ts, n = O.time_grid(cfg)
+    tab = StepTables(PSLDSchedule(cfg), torch.from_numpy(ts), n, "sscs_sde", True, 1e-3, merge_noise=True)
+    halves = [s.half_step(float(ts[i]), float(ts[i + 1] - ts[i]) / 2) for i in range(n)]
+    err_a, err_s, size_s = [], [], []
+    for i in range(n):
+        r = tab.sscs[i]
+        hb = r.half_b
+        a = np.array([[hb.a_xx, hb.a_xm], [hb.a_mx, hb.a_mm]])
+        lt = np.array([[hb.c11, hb.c12], [hb.c21, hb.c22]])
+        if i + 1 < n:
+            a_ref, S = _merge_ref(halves[i], halves[i + 1])
+            assert hb.c12 == 0.0 and hb.c11 > 0 and hb.c22 > 0
+        else:
+            a_ref = np.array(halves[i][0]).reshape(2, 2)
+            l_ref = np.array(halves[i][1]).reshape(2, 2)
+            S = l_ref @ l_ref.T
+        err_a.append(float(np.abs(a - a_ref).max() / np.abs(a_ref).max()))
+        err_s.append(float(np.abs(lt @ lt.T - S).max()))
+        size_s.append(float(np.abs(S).max()))
+        np.testing.assert_allclose([r.half_a.a_xx, r.half_a.c11, r.half_a.c21, r.half_a.c22],
+                                   [halves[i][0][0], *np.array(halves[i][1])[[0, 2, 3]]], rtol=1e-10)
+    err_s, size_s = np.array(err_s), np.array(size_s)
+    worst_a, worst_s = max(err_a), float(err_s.max() / size_s.max())
+    # per row: the oracle (math.exp) and the tables (torch.exp) evaluate the half-step variance
+    # separately; at the smallest quadratic-stride steps its bracket cancels to ~2e-13 of the row
+    worst_row = float((err_s / size_s).max())
+    print(f"merged rows: A {worst_a:.2e}, covariance {worst_s:.2e} of max|S| ({worst_row:.2e} per row)")
+    assert worst_a <= 1e-13 and worst_s <= 1e-13 and worst_row <= 1e-11, (worst_a, worst_s, worst_row)
